@@ -2,7 +2,7 @@
 """bench.py - headline benchmark of the render hot path (BASELINE.json: Mrays/s, all bounces; ms/frame at 2800x2240, 64 spp).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload mesh100k|mesh1m|mesh5m|bundled|cornell|mesh1m4k]
-                    [--accel bvh|lbvh|grid|emu] [--scaling weak|strong] [--impl ptap|reference]
+                    [--accel bvh|lbvh|grid|emu] [--scaling weak|strong] [--impl ptap|reference] [--dump-outputs DIR]
 
 A "step" is one whole frame of the workload: Renderer::renderLoop for `spp` iterations (ray generation, closest hit,
 shading + compaction, film accumulation for every bounce).  Rays = rays actually traced, summed over closest-hit launches
@@ -31,6 +31,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the tree may be read-only: the benchmark writes nothing into it
 
 GOLDEN_SCENE = os.path.join(ROOT, "tests", "golden", "bundled_scene.npz")
 DIFFUSE, EMISSIVE = 0, 4            # Primitive.h:70-79
@@ -213,13 +214,29 @@ def reference_gpu_arm(device_index: int):
     return out
 
 
+# ------------------------------------------------------------------------------------------------ outputs
+
+DUMP_PIXELS = 1 << 22               # 48 MB of float32 RGB: films above this are sampled, so that a dump stays under 64 MB
+
+
+def dump_outputs(out_dir: str, film: np.ndarray):
+    """--dump-outputs: the film of the last timed step (the un-normalised H x W x 3 float32 sum Renderer.film() returns) as
+    out_dir/film.npy, so that two builds can be compared output for output.  A film of more than DUMP_PIXELS pixels is written as
+    the pixels of one fixed sample (seed 0, ascending pixel index, DUMP_PIXELS x 3): the same pixels for every build at one resolution."""
+    os.makedirs(out_dir, exist_ok=True)
+    H, W, _ = film.shape
+    if H * W > DUMP_PIXELS:
+        film = film.reshape(-1, 3)[np.sort(np.random.default_rng(0).choice(H * W, DUMP_PIXELS, replace=False))]
+    np.save(os.path.join(out_dir, "film.npy"), film)
+
+
 # ------------------------------------------------------------------------------------------------ main
 
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=3)
-    ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--warmup", type=int, default=3, help="untimed steps before the timed ones: at least 3 (1 for --impl reference); the JSON reports the count run")
     ap.add_argument("--impl", default="ptap", choices=["ptap", "reference"])
     ap.add_argument("--workload", default="mesh1m", choices=sorted(WORKLOADS))
     ap.add_argument("--spp", type=int, default=0, help="override samples per pixel of the workload")
@@ -229,7 +246,13 @@ def main():
     ap.add_argument("--no-cache", action="store_true", help="disable the first-hit cache (Renderer.cpp:594-613)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the second BASELINE metric (bundled 2800x2240), the lbvh end-to-end line and the reference's GPU kernels")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the film of the last timed step to DIR/film.npy (float32; a fixed pixel sample above 4 Mpixels)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ptap":
+        ap.error("--dump-outputs writes the film of --impl ptap")
+    warmup = max(args.warmup, 3 if args.impl == "ptap" else 1)
 
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1")); local = int(os.environ.get("LOCAL_RANK", "0"))
     W, H, spp, depth, desc = WORKLOADS[args.workload]
@@ -246,7 +269,7 @@ def main():
         arrays = reference_arrays(args.workload)
         sw, sh = sample_size(W, H, 140_000)
         ITERS = 8
-        for _ in range(max(args.warmup, 1)):
+        for _ in range(warmup):
             cpu_reference_arm(arrays, depth, sw, sh, 1)
         vals, rays_total, t_total = [], 0, 0.0
         for _ in range(args.steps):
@@ -255,7 +278,7 @@ def main():
         value = rays_total / t_total / 1e6
         sample = f"{sw}x{sh} x {ITERS} iterations per step of the {args.workload} scene, full bounce loop, reference 25^3 grid, no first-hit cache"
         print(json.dumps({"impl": "reference", "metric": metric, "value": round(value, 4), "unit": unit, "n_gpus": args.gpus, "steps": args.steps,
-                          "warmup": args.warmup, "ms_per_step": round(t_total / args.steps * 1e3, 3), "higher_is_better": True, "scaling": args.scaling,
+                          "warmup": warmup, "ms_per_step": round(t_total / args.steps * 1e3, 3), "higher_is_better": True, "scaling": args.scaling,
                           "vs_baseline": None, "dtype": "f32", "data": "synthetic",
                           "config": {"workload": args.workload, "description": desc, "resolution": [W, H], "spp": spp, "depth": depth},
                           "cpu_baseline": {"value": round(value, 4), "unit": unit, "cores": cores, "kind": kind, "sample": sample},
@@ -334,7 +357,7 @@ def main():
     if world > 1 and reduce_how is None:
         film_t = multi_gpu.film_tensor(r)      # zero-copy torch view of the library's film buffer
 
-    for _ in range(max(args.warmup, 3)):
+    for _ in range(warmup):
         step()
     barrier()
     sampler = ClockSampler(dev)
@@ -353,6 +376,8 @@ def main():
     barrier()
     t_wall = time.perf_counter() - t_wall0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, r.film())      # N > 1: rank 0's film holds the reduced frame
 
     def over_ranks(t_rank, n_rank):
         if world == 1:
@@ -513,7 +538,7 @@ def main():
     par = f"sample-partition x{world}"
     if world > 1:
         par += " + 1 NCCL reduce of the film (" + ("ptap_reduce: ncclReduce through the library's C ABI" if reduce_how else "torch.distributed.reduce") + ")"
-    out = {"metric": metric, "value": round(value, 2), "unit": unit, "n_gpus": world, "steps": args.steps, "warmup": max(args.warmup, 3),
+    out = {"metric": metric, "value": round(value, 2), "unit": unit, "n_gpus": world, "steps": args.steps, "warmup": warmup,
            "ms_per_step": round(t_max / args.steps * 1e3, 3), "higher_is_better": True, "scaling": args.scaling, "vs_baseline": None,
            "dtype": "f32", "data": "synthetic",
            "config": {"workload": args.workload, "description": desc, "resolution": [W, H], "spp_per_gpu": it1 - it0, "spp_total": total_spp, "depth": depth,

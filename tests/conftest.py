@@ -38,16 +38,6 @@ def port():
 
 
 @pytest.fixture(scope="session")
-def ref():
-    """The reference's own sources compiled for the host (oracle/_ref); skipped where it was never built."""
-    from oracle import ref as r
-    if not r.available():
-        pytest.skip("oracle/_ref/libptap_ref.so not built (needs /root/reference): golden fixtures cover this machine")
-    r.lib()
-    return r
-
-
-@pytest.fixture(scope="session")
 def golden_scene():
     z = np.load(os.path.join(GOLDEN, "bundled_scene.npz"))
     return {k: z[k] for k in z.files}

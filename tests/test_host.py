@@ -234,10 +234,12 @@ def test_config_txt_parser(libptap, tmp_path):
 
 
 def test_reference_config_txt_parses(libptap, tmp_path):
-    """The reference's own sample file, when the tree is mounted (its MESH path points at a file that is not bundled)."""
-    src = "/root/reference/PathTracerAP/Config.txt"
+    """The reference's own sample file (its MESH path points at a file that is not bundled).  The file belongs to the original
+    PathTracerAP sources, which this repository does not carry: the test runs where PTAP_REFERENCE points at a checkout of them."""
+    from oracle.ref import REFERENCE_ROOT
+    src = os.path.join(REFERENCE_ROOT, "PathTracerAP", "Config.txt")
     if not os.path.exists(src):
-        pytest.skip("reference tree not mounted")
+        pytest.skip("needs the original PathTracerAP sources (PTAP_REFERENCE), which are not part of this repository")
     text = open(src).read()
     from pathtracerap_b200 import PtapError, Scene
     cfg = tmp_path / "Config.txt"

@@ -1,14 +1,25 @@
 """The C restatement (oracle/ptap_oracle.c) against vectors dumped from the reference's own code (tools/make_golden.py).
 These run on any machine: they need neither /root/reference nor a GPU."""
 import hashlib
+import os
 
 import numpy as np
+import pytest
+
+from conftest import GOLDEN
+from oracle import live_scenes, ref
 
 FLOAT_MAX = np.float32(9999999.0)
 
 
 def sha(a):
     return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
+
+
+@pytest.fixture(scope="module")
+def golden_live():
+    z = np.load(os.path.join(GOLDEN, "live_scenes.npz"))
+    return {k: z[k] for k in z.files}
 
 
 def test_hash_and_rng_known_answers(port, golden_kat):
@@ -157,21 +168,18 @@ def test_films_golden_r1(port, oracle_scene, golden_films):
     w2.close()
 
 
-def test_bmp_writer_vs_compiled_reference(ref, port, golden_scene, tmp_path):
+def test_bmp_writer_vs_compiled_reference(port, golden_scene, golden_live, tmp_path):
     """Renderer::renderImage (Renderer.cpp:15-63) of the compiled reference, run on its own film, against the port's writer on the same film:
-    the two files must be byte-identical (header, row order, channel order, (char) truncation)."""
-    g = golden_scene
-    rscene = ref.RefScene.from_arrays(g["models"], g["meshes"], g["vertices"], g["triangles"])
-    W, H, iters = 96, 64, 3
-    rr = ref.RefRenderer(rscene, W, H, 5)
-    rr.init_image()
-    for it in range(iters):
-        rr.run_iteration(it)
-    film = rr.image()
-    d = tmp_path / "refout"; d.mkdir()
-    rr.write_bmp(str(d), iters)
-    rr.close(); rscene.close()
-    want = (d / "Render.bmp").read_bytes()
+    the two files must be byte-identical (header, row order, channel order, (char) truncation).  The film and the file are stored in
+    tests/golden/live_scenes.npz (its `source` entry names what wrote them); where oracle/_ref is built, the reference renders and
+    writes them again live and must match them too."""
+    W, H, depth, iters = live_scenes.BMP
+    film, want = golden_live["bmp_film"], golden_live["bmp_bytes"].tobytes()
+    if ref.available():
+        rfilm, rbytes = live_scenes.reference_bmp(golden_scene)
+        assert np.array_equal(rfilm, film) and rbytes == want
+    _, pfilm = live_scenes.Port().frame(port.OracleScene(golden_scene), W, H, depth, iters, 0)
+    assert np.array_equal(pfilm, film)
     port.write_bmp(film, iters, tmp_path / "port.bmp")
     got = (tmp_path / "port.bmp").read_bytes()
     assert len(want) == 54 + 3 * W * H
@@ -211,93 +219,28 @@ def test_committed_render_bmp(port, oracle_scene, golden_render_bmp):
     assert psnr >= 39.0
 
 
-def _random_instances(golden_scene, n, seed):
-    """n instances of the three bundled meshes under random rotations, non-uniform scales and translations (column-major matrices)."""
-    from oracle.port import MODEL
-    rs = np.random.RandomState(seed)
-    models = np.zeros(n, MODEL)
-    for k in range(n):
-        a = rs.randn(3); a /= np.linalg.norm(a)
-        t = np.deg2rad(rs.uniform(0, 360)); c, s = np.cos(t), np.sin(t)
-        K = np.array([[0, -a[2], a[1]], [a[2], 0, -a[0]], [-a[1], a[0], 0]])
-        R = np.eye(3) * c + s * K + (1 - c) * np.outer(a, a)
-        M = np.eye(4)
-        M[:3, :3] = R @ np.diag(rs.uniform(0.02, 0.12, 3) * (0.3 if k % 3 == 0 else 1.0))
-        M[:3, 3] = rs.uniform(-500, 500, 3) + [0, 0, 300]
-        models[k]["mesh_index"] = k % 3
-        models[k]["model_to_world"] = M.T.astype(np.float32).reshape(16)
-        models[k]["world_to_model"] = np.linalg.inv(M.astype(np.float32).astype(np.float64)).T.astype(np.float32).reshape(16)
-        models[k]["mat"]["type"] = [0, 6, 5, 2, 4][k % 5]          # DIFFUSE, METAL, COAT, REFLECTIVE, EMISSIVE
-        models[k]["mat"]["color"] = rs.uniform(0.2, 0.99, 3)
-    return models
-
-
-def test_port_equals_compiled_reference_on_other_scenes(ref, port, golden_scene):
-    """The golden fixtures pin the C restatement on the bundled scene.  Where the reference itself is built (oracle/_ref), the two are
-    also compared LIVE on scenes the fixtures do not hold - random rotated / non-uniformly scaled instances, all five material branches -
-    for the grid build, both trace tiers on random rays, and two whole iterations of the wavefront: bit-equal everywhere."""
-    g = golden_scene
-    for n, seed in ((24, 3), (7, 8)):
-        models = _random_instances(g, n, seed)
-        rscene = ref.RefScene.from_arrays(models, g["meshes"], g["vertices"], g["triangles"])
-        ra = rscene.arrays()
-        pscene = port.OracleScene({"models": models, "meshes": g["meshes"], "vertices": g["vertices"], "triangles": g["triangles"]})
-        pa = pscene.arrays()
-        for k in ("grids", "voxels", "refs"):
-            assert ra[k].tobytes() == pa[k].tobytes(), f"{k} differ ({n} instances)"
-        W, H, depth = 64, 48, 5
-        rr = ref.RefRenderer(rscene, W, H, depth)
-        rs = np.random.RandomState(seed)
-        o = rs.uniform(-700, 700, (20000, 3)) + [0, 0, 300]
-        d = rs.uniform(-400, 400, (20000, 3)) + [0, 0, 300] - o
-        d[:200, 0] = 0.0
-        rays = np.concatenate([o, d], 1).astype(np.float32)
+def _check_live(scene_list, golden_live, min_hit):
+    """The C restatement - and, where oracle/_ref is built, the compiled reference itself - against the stored outputs."""
+    impls = [("port", live_scenes.Port())] + ([("reference", live_scenes.Reference())] if ref.available() else [])
+    for name, impl in impls:
+        got = live_scenes.outputs(impl, scene_list)
+        for k, v in got.items():
+            want = golden_live[k]
+            assert v.dtype == want.dtype and v.shape == want.shape and v.tobytes() == want.tobytes(), f"{name}: {k} differs"
+    for key, *_ in scene_list:
         for mode in (0, 1):
-            a, b = rr.trace_rays(rays, mode), pscene.trace(rays, mode)
-            assert np.array_equal(a["model"], b["model"]) and np.array_equal(a["tri"], b["tri"]), f"mode {mode}: ids differ"
-            hit = a["model"] >= 0
-            assert hit.mean() > 0.05
-            for f in ("dist", "u", "v"):
-                assert np.array_equal(a[f][hit], b[f][hit]), f"mode {mode}: {f} differs"
-        pw = port.OracleWavefront(pscene, W, H, depth)
-        rr.init_image(); pw.init_image()
-        for it in range(2):
-            assert rr.run_iteration(it) == pw.run_iteration(it)
-        assert np.array_equal(rr.image(), pw.image())
-        # the same two iterations at tier R1 (BVH film parity rests on this mode of the port)
-        pw1 = port.OracleWavefront(pscene, W, H, depth, mode=1)
-        rr.init_image(); pw1.init_image()
-        for it in range(2):
-            assert rr.run_iteration(it, mode=1) == pw1.run_iteration(it)
-        assert np.array_equal(rr.image(), pw1.image())
-        rr.close(); pw.close(); pw1.close(); rscene.close()
+            assert (golden_live[f"{key}_r{mode}_model"] >= 0).mean() > min_hit
 
 
-def test_port_equals_compiled_reference_on_a_dense_mesh(ref, port, libptap):
-    """Same live comparison on the kind of mesh the throughput workloads use: a displaced icosphere (5120 triangles; the host-side
+def test_port_equals_compiled_reference_on_other_scenes(port, golden_scene, golden_live):
+    """The golden fixtures pin the C restatement on the bundled scene.  Here it is compared on scenes they do not hold - random rotated /
+    non-uniformly scaled instances, all five material branches - for the grid build, both trace tiers on random rays, and two whole
+    iterations of the wavefront at both tiers (BVH film parity rests on tier R1 of the port): bit-equal to the outputs stored in
+    tests/golden/live_scenes.npz, and, where oracle/_ref is built, the reference's own outputs must equal them as well."""
+    _check_live(live_scenes.scenes(golden_scene, ("instances",)), golden_live, 0.05)
+
+
+def test_port_equals_compiled_reference_on_a_dense_mesh(port, libptap, golden_scene, golden_live):
+    """Same comparison on the kind of mesh the throughput workloads use: a displaced icosphere (5120 triangles; the host-side
     generator of libptap needs no GPU), three instances, so that voxels hold many references and the 3D-DDA early exit matters."""
-    from pathtracerap_b200 import DIFFUSE, Scene
-    s = Scene.empty()
-    mi = s.add_icosphere(4, radius=1000.0, displacement=0.05, seed=2)
-    for k, (tr, sc) in enumerate([((0, 0, 0), 0.2), ((260, 40, -120), 0.12), ((-240, -60, 80), 0.3)]):
-        s.add_model(mi, translate=tr, rotate_y_degrees=25.0 * k, scale=(sc, sc * (1 + 0.3 * k), sc), material=DIFFUSE, color=(0.7, 0.6, 0.5))
-    a = s.arrays()
-    assert len(a["triangles"]) == 5120
-    rscene = ref.RefScene.from_arrays(a["models"], a["meshes"], a["vertices"], a["triangles"])
-    pscene = port.OracleScene({k: a[k] for k in ("models", "meshes", "vertices", "triangles")})
-    ra, pa = rscene.arrays(), pscene.arrays()
-    for k in ("grids", "voxels", "refs"):
-        assert ra[k].tobytes() == pa[k].tobytes(), f"{k} differ"
-    rr = ref.RefRenderer(rscene, 32, 32, 5)
-    rs = np.random.RandomState(4)
-    o = rs.uniform(-600, 600, (6000, 3))
-    d = rs.uniform(-250, 250, (6000, 3)) - o
-    rays = np.concatenate([o, d], 1).astype(np.float32)
-    for mode in (0, 1):
-        x, y = rr.trace_rays(rays, mode), pscene.trace(rays, mode)
-        assert np.array_equal(x["model"], y["model"]) and np.array_equal(x["tri"], y["tri"])
-        hit = x["model"] >= 0
-        assert hit.mean() > 0.3
-        for f in ("dist", "u", "v"):
-            assert np.array_equal(x[f][hit], y[f][hit])
-    rr.close(); rscene.close()
+    _check_live(live_scenes.scenes(golden_scene, ("dense",)), golden_live, 0.3)

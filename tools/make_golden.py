@@ -4,7 +4,13 @@
 Run in the build container, where /root/reference exists:   python tools/make_golden.py
 The reference ships no golden vectors of its own (SURVEY.md 4); these files are outputs of ITS code
 (Renderer.cpp / Scene.cpp through oracle/ref_harness.cpp) and travel to the GPU box, where /root/reference
-does not exist.  Nothing here comes from this repository's own kernels or from the C restatement.
+does not exist.  Nothing here comes from this repository's own kernels.
+
+    python tools/make_golden.py live_scenes
+
+writes only tests/golden/live_scenes.npz (oracle/live_scenes.py): from the compiled reference where oracle/_ref is built,
+otherwise from the C restatement, which tests/test_oracle_golden.py compares with the compiled reference live, bit for bit,
+wherever that is built.  The file's `source` entry names which of the two wrote it.
 """
 import hashlib
 import os
@@ -14,7 +20,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-from oracle import ref  # noqa: E402
+from oracle import live_scenes, port, ref  # noqa: E402
 
 OUT = os.path.join(ROOT, "tests", "golden")
 os.makedirs(OUT, exist_ok=True)
@@ -31,7 +37,30 @@ def cornell_models(models):
     return m
 
 
+def write_live_scenes():
+    g = np.load(os.path.join(OUT, "bundled_scene.npz"))
+    g = {k: g[k] for k in ("models", "meshes", "vertices", "triangles")}
+    if ref.available():
+        source = "the compiled reference (oracle/_ref)"
+        out = live_scenes.outputs(live_scenes.Reference(), live_scenes.scenes(g))
+        film, bmp = live_scenes.reference_bmp(g)
+    else:
+        source = "the C restatement (oracle/ptap_oracle.c), held bit-equal to the compiled reference wherever oracle/_ref is built"
+        out = live_scenes.outputs(live_scenes.Port(), live_scenes.scenes(g))
+        W, H, depth, iters = live_scenes.BMP
+        _, film = live_scenes.Port().frame(port.OracleScene(g), W, H, depth, iters, 0)
+        path = os.path.join(OUT, "_bmp.tmp")
+        port.write_bmp(film, iters, path)
+        bmp = open(path, "rb").read(); os.remove(path)
+    np.savez_compressed(os.path.join(OUT, "live_scenes.npz"), source=np.array(source), bmp_film=film,
+                        bmp_bytes=np.frombuffer(bmp, np.uint8), **out)
+    print("live_scenes.npz from", source, os.path.getsize(os.path.join(OUT, "live_scenes.npz")), "bytes")
+
+
 def main():
+    if sys.argv[1:] == ["live_scenes"]:
+        write_live_scenes()
+        return
     scene = ref.RefScene.builtin()
     A = scene.arrays()
     np.savez_compressed(os.path.join(OUT, "bundled_scene.npz"), models=A["models"], meshes=A["meshes"], vertices=A["vertices"],
@@ -143,6 +172,7 @@ def main():
     rc.init_image()
     print("cornell 512x512 iteration 0 active:", rc.run_iteration(0))
     rc.close()
+    write_live_scenes()
     for f in sorted(os.listdir(OUT)):
         print(f, os.path.getsize(os.path.join(OUT, f)))
 
