@@ -34,7 +34,8 @@
 extern "C" {
 #endif
 
-#define PTAP_VERSION 2      /* 2: PtapBvhNode carries node-local offsets; ptap_render_probe, ptap_reduce*, stamps */
+#define PTAP_VERSION 3      /* 2: PtapBvhNode carries node-local offsets; ptap_render_probe, ptap_reduce*, stamps
+                               3: ray queries on device buffers, ptap_query_closest / ptap_query_occluded */
 
 enum {
     PTAP_OK = 0,
@@ -276,6 +277,23 @@ int ptap_nccl_init(ptap_ctx* ctx, const void* id128, int32_t nranks, int32_t ran
 int ptap_reduce(ptap_ctx* ctx, int32_t root);
 int ptap_nccl_finalize(ptap_ctx* ctx);
 void* ptap_stream(ptap_ctx* ctx);                                  /* cudaStream_t of the context */
+
+/* ---- ray queries on device buffers (DESIGN.md 4.8) ----------------------------------------------------------------------------------
+ * Embree's rtcIntersect / rtcOccluded for rays already in GPU memory.  Every pointer is a DEVICE (or managed) pointer on the context's
+ * device; org and dir each hold n x 4 floats, 16-byte aligned: org[i] = (ox, oy, oz, unused), dir[i] = (dx, dy, dz, L_i).  Origin and
+ * direction are in world space, d need not be normalised, and distances are WORLD distances, length(hit - o) (Renderer.cpp:388-391).
+ *   ptap_query_closest:  hits[i] = what ptap_trace returns for (o, d) under the current accel, bit for bit (tier R0 for the grid modes,
+ *                        R1 for the BVH modes); dir[i].w is not read.
+ *   ptap_query_occluded: occluded[i] = (closest.model >= 0 && closest.dist < L_i) in binary32 (1 / 0): L = +inf is "any hit", a NaN L
+ *                        gives 0.  Under PTAP_ACCEL_BVH / BVH_DEVICE an any-hit traversal stops at the first hit that provably decides
+ *                        the answer; the grid modes compute the closest hit (their walk can miss hits, so no early exit is exact) and compare.
+ * stream: NULL = ptap_stream(ctx); otherwise the work is ordered after everything already enqueued on `stream`, and `stream` is ordered
+ * after the query (event record + wait both ways).  The call returns after enqueueing: no host synchronisation.  Work already enqueued on
+ * ptap_stream(ctx) (a render) runs first; the queries use scratch of their own and never change the film.  Rays are processed in chunks
+ * of 2^22; the scratch (one chunk: 16 B per ray, 24 B for closest, plus 156 B per ray + 33 MB under PTAP_ACCEL_GRID_EMULATED) is kept
+ * for later calls.  Bad pointers (host memory, another device, misaligned) give PTAP_E_INVALID naming the argument; n == 0 is a no-op. */
+int ptap_query_closest(ptap_ctx* ctx, const float* org, const float* dir, int32_t n, PtapHit* hits, void* stream);
+int ptap_query_occluded(ptap_ctx* ctx, const float* org, const float* dir, int32_t n, uint8_t* occluded, void* stream);
 
 /* ---- parity entry points (what BASELINE.json's contract measures) ------------------------- */
 

@@ -104,6 +104,12 @@ struct ptap_ctx {
     unsigned long long* d_stamps = nullptr;   // PTAP_FLAG_STAMP: (start, end) %globaltimer words of the closest-hit launches of the last render call
     int stamps_used = 0;
     bool render_pending = false;
+    // ptap_query_*: scratch of their own (never an arena a render uses), the events that order them with the caller's stream, and
+    // whether BVH occlusion takes the any-hit traversal.  Not an option of the ABI: an internal switch for the A/B measurement of
+    // tools/bench_queries.py (PTAP_QUERY_ANYHIT=0 in the environment at ptap_create: closest hit + compare, the same answers)
+    Arena query_arena;
+    cudaEvent_t e_qin = nullptr, e_qout = nullptr;
+    bool query_anyhit = true;
     std::string err;
 };
 
@@ -582,6 +588,10 @@ int ptap_create(int device, size_t arena_bytes, ptap_ctx** out)
     ctx->emu_replay_ctas = std::max(1, envInt("PTAP_EMU_REPLAY_CTAS", 6));     // CTAs per SM of k_emu_tail (k_emu_setup: twice as many); tuning only
     ctx->emu_walk_ctas = std::max(1, envInt("PTAP_EMU_WALK_CTAS", 2));
     ctx->sc.emu_refill = std::min(32, std::max(1, envInt("PTAP_EMU_REFILL", 8)));
+    ctx->query_anyhit = envInt("PTAP_QUERY_ANYHIT", 1) != 0;
+    if (cudaEventCreateWithFlags(&ctx->e_qin, cudaEventDisableTiming) != cudaSuccess || cudaEventCreateWithFlags(&ctx->e_qout, cudaEventDisableTiming) != cudaSuccess) {
+        ptap_destroy(ctx); return PTAP_E_NOMEM;
+    }
     if (arena_bytes) {                                          // caller-sized arena: split 1/4 scene, 3/4 frame
         if (ctx->scene_arena.reserve(arena_bytes / 4) != cudaSuccess || ctx->frame_arena.reserve(arena_bytes - arena_bytes / 4) != cudaSuccess) {
             ptap_destroy(ctx); return PTAP_E_NOMEM;
@@ -599,7 +609,8 @@ void ptap_destroy(ptap_ctx* ctx)
     for (int l = 1; l < kMaxLanes; ++l) if (ctx->streams[l]) { cudaStreamSynchronize(ctx->streams[l]); cudaStreamDestroy(ctx->streams[l]); }
     for (cudaEvent_t e : {ctx->e_fork, ctx->e_cache}) if (e) cudaEventDestroy(e);
     for (int l = 0; l < kMaxLanes; ++l) { if (ctx->e_join[l]) cudaEventDestroy(ctx->e_join[l]); if (ctx->e_gather[l]) cudaEventDestroy(ctx->e_gather[l]); }
-    ctx->scene_arena.release(); ctx->frame_arena.release(); ctx->scratch.release(); ctx->emu_arena.release();
+    ctx->scene_arena.release(); ctx->frame_arena.release(); ctx->scratch.release(); ctx->emu_arena.release(); ctx->query_arena.release();
+    for (cudaEvent_t e : {ctx->e_qin, ctx->e_qout}) if (e) cudaEventDestroy(e);
     if (ctx->gd_cells) cudaFree(ctx->gd_cells);
     if (ctx->d_tri_box) cudaFree(ctx->d_tri_box);
     if (ctx->gd_refs) cudaFree(ctx->gd_refs);
@@ -1176,6 +1187,82 @@ static int traceImpl(ptap_ctx* ctx, const float* rays_od, int32_t n, PtapHit* ou
 
 int ptap_trace(ptap_ctx* ctx, const float* rays_od, int32_t n, PtapHit* out) { return traceImpl(ctx, rays_od, n, out, nullptr); }
 int ptap_trace_count(ptap_ctx* ctx, const float* rays_od, int32_t n, PtapHit* out, int32_t* counts) { return traceImpl(ctx, rays_od, n, out, counts); }
+
+// ---- ray queries on device buffers (DESIGN.md 4.8) ---------------------------------------------------------------
+
+static int checkQueryPtr(ptap_ctx* ctx, const char* call, const char* arg, const void* p, size_t align)
+{
+    if (!p) return fail(ctx, PTAP_E_INVALID, "%s: %s is NULL", call, arg);
+    if ((uintptr_t)p % align) return fail(ctx, PTAP_E_INVALID, "%s: %s is not %zu-byte aligned", call, arg, align);
+    cudaPointerAttributes a{};
+    if (cudaPointerGetAttributes(&a, p) != cudaSuccess) {
+        cudaGetLastError();                                     // clear the sticky-free error of the failed query
+        return fail(ctx, PTAP_E_INVALID, "%s: %s is not a pointer CUDA knows", call, arg);
+    }
+    if (a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged) return fail(ctx, PTAP_E_INVALID, "%s: %s is not device or managed memory", call, arg);
+    if (a.device != ctx->device) return fail(ctx, PTAP_E_INVALID, "%s: %s is on device %d, the context on device %d", call, arg, a.device, ctx->device);
+    return PTAP_OK;
+}
+
+// One implementation for both queries: validation, stream ordering (the caller's stream -> context stream -> the caller's stream), and chunks
+// of at most kQueryChunk rays through the query arena, which is sized for one chunk and reused by every later call.
+static int queryImpl(ptap_ctx* ctx, const char* call, const float* org, const float* dir, int32_t n, PtapHit* hits, uint8_t* occluded, void* stream)
+{
+    constexpr int kQueryChunk = 1 << 22;
+    if (!ctx) return PTAP_E_INVALID;
+    if (n < 0) return fail(ctx, PTAP_E_INVALID, "%s: n = %d", call, n);
+    if (n == 0) return PTAP_OK;
+    if (!ctx->have_scene) return fail(ctx, PTAP_E_STATE, "%s: no scene uploaded", call);
+    if ((ctx->accel == PTAP_ACCEL_GRID_COMPAT || ctx->accel == PTAP_ACCEL_GRID_EMULATED) && !ctx->have_grid) return fail(ctx, PTAP_E_STATE, "%s: no grid in the uploaded scene", call);
+    CK(cudaSetDevice(ctx->device));
+    { const int rc = checkQueryPtr(ctx, call, "org", org, 16); if (rc) return rc; }
+    { const int rc = checkQueryPtr(ctx, call, "dir", dir, 16); if (rc) return rc; }
+    { const int rc = hits ? checkQueryPtr(ctx, call, "hits", hits, alignof(PtapHit)) : checkQueryPtr(ctx, call, "occluded", occluded, 1); if (rc) return rc; }
+    const bool emulated = ctx->accel == PTAP_ACCEL_GRID_EMULATED;
+    const bool anyhit = occluded && ctx->query_anyhit && (ctx->accel == PTAP_ACCEL_BVH || ctx->accel == PTAP_ACCEL_BVH_DEVICE);
+    const size_t chunk = std::min<size_t>((size_t)n, kQueryChunk);
+    const size_t need = Arena::need(chunk, sizeof(float4)) + (hits ? Arena::need(chunk, sizeof(float2)) : 0) + Arena::need(1, sizeof(FrameState)) +
+                        (emulated ? emuArenaNeed(ctx, chunk) : 0) + 4096;
+    cudaStream_t S = ctx->stream, U = (cudaStream_t)stream;
+    if (need > ctx->query_arena.cap) {
+        CK(cudaStreamSynchronize(S));                           // earlier queries may still read the arena being replaced
+        CK(ctx->query_arena.reserve(need));
+    } else ctx->query_arena.used = 0;
+    Arena& A = ctx->query_arena;
+    float4* hit = A.alloc<float4>(chunk);
+    float2* uv = hits ? A.alloc<float2>(chunk) : nullptr;
+    FrameState* st = A.alloc<FrameState>(1);
+    const EmuBuf emu = emulated ? emuFromArena(ctx, A, chunk) : EmuBuf{};
+    if (!ctx->grid_trace) ctx->grid_trace = traceGridSize(ctx);
+    if (U && U != S) { CK(cudaEventRecord(ctx->e_qin, U)); CK(cudaStreamWaitEvent(S, ctx->e_qin, 0)); }
+    const float4* O = reinterpret_cast<const float4*>(org);
+    const float4* D = reinterpret_cast<const float4*>(dir);
+    for (size_t off = 0; off < (size_t)n; off += chunk) {
+        const int m = (int)std::min(chunk, (size_t)n - off);
+        CK(cudaMemsetAsync(st, 0, sizeof(FrameState), S));    // arms the work-stealing cursor
+        if (hits) {                                             // what ptap_trace launches, on device buffers
+            launchTrace(ctx, st, O + off, D + off, hit, uv, nullptr, 0, m, emu, false, S);
+            launchResolveHits(ctx->sc, O + off, D + off, hit, uv, m, hits + off, S);
+        } else {
+            if (anyhit) launchTraceBvhAny(ctx->sc, O + off, D + off, hit, st, m, ctx->grid_trace, S);
+            else launchTrace(ctx, st, O + off, D + off, hit, nullptr, nullptr, 0, m, emu, false, S);   // grid modes: R0 may miss hits, no early exit
+            launchResolveOccluded(ctx->sc, O + off, D + off, hit, m, occluded + off, S);
+        }
+    }
+    CK(cudaGetLastError());
+    if (U && U != S) { CK(cudaEventRecord(ctx->e_qout, S)); CK(cudaStreamWaitEvent(U, ctx->e_qout, 0)); }
+    return PTAP_OK;
+}
+
+int ptap_query_closest(ptap_ctx* ctx, const float* org, const float* dir, int32_t n, PtapHit* hits, void* stream)
+{
+    return queryImpl(ctx, "query_closest", org, dir, n, hits, nullptr, stream);
+}
+
+int ptap_query_occluded(ptap_ctx* ctx, const float* org, const float* dir, int32_t n, uint8_t* occluded, void* stream)
+{
+    return queryImpl(ctx, "query_occluded", org, dir, n, nullptr, occluded, stream);
+}
 
 int ptap_shade(ptap_ctx* ctx, const PtapPathIn* paths, int32_t n, int32_t iter, int32_t remaining, PtapPathOut* out, int32_t* order, int32_t* n_alive)
 {

@@ -9,6 +9,7 @@ namespace ptap {
 constexpr float kEpsilon = 0.005f;          // Config.h:4
 constexpr float kFloatMax = 9999999.0f;     // Config.h:5
 constexpr float kFloatMin = -9999990.0f;    // Config.h:6
+constexpr int kAnyOccluded = -2;            // model field of an any-hit record whose ray retired as occluded (k_trace_bvh<.., ANY>)
 constexpr int kMaxDepth = 16;               // rounds per iteration the context reserves state for
 constexpr int kBigHits = 108;               // k_emu_full: further hits of a (ray, model) kept per thread in global memory (128 with the 20 in shared memory)
 constexpr int kEmuHits = 8;                 // PTAP_ACCEL_GRID_EMULATED: hits of a (ray, model) that are kept for the replay of the walk

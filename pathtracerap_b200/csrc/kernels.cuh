@@ -61,6 +61,8 @@ int traceGridOccupancy();
 void launchTraceBvh(const SceneDev& sc, const float4* O, const float4* D, float4* hit, float2* uv, int4* counts, bool count_totals,
                     FrameState* st, int round, int n_fixed, int grid, cudaStream_t stream, unsigned long long* stamp = nullptr);
 int traceBvhOccupancy();
+// the any-hit traversal of ptap_query_occluded over rays [0, n): L = D[i].w; records for launchResolveOccluded
+void launchTraceBvhAny(const SceneDev& sc, const float4* O, const float4* D, float4* hit, FrameState* st, int n, int grid, cudaStream_t stream);
 
 // bvh_device.cu
 size_t deviceBvhScratchBytes(int ntris);
@@ -81,6 +83,8 @@ void launchShade(const SceneDev& sc, const WaveDev& wv, int round, int in_buf, c
                  int iter_fixed, int* slot_pos, int grid, cudaStream_t stream);
 int shadeOccupancy();
 void launchResolveHits(const SceneDev& sc, const float4* O, const float4* D, const float4* hit, const float2* uv, int n, PtapHit* out, cudaStream_t stream);
+// occluded[i] = closest hit of ray i nearer than L = D[i].w, from closest-hit records or any-hit ones (model kAnyOccluded: occluded)
+void launchResolveOccluded(const SceneDev& sc, const float4* O, const float4* D, const float4* hit, int n, uint8_t* occluded, cudaStream_t stream);
 void launchSetIter(FrameState* st, int iter, cudaStream_t stream);
 void launchFilmAdd(float* film, const float* add, size_t n, cudaStream_t stream);
 void launchResolveBmp(const float* film, size_t nvalues, float div, unsigned char* out, cudaStream_t stream);

@@ -21,6 +21,9 @@
 //  * work stealing: each warp takes batches of consecutive rays from a device-side cursor (one atomic per batch).
 //  * cross-instance pruning: once some instance reported a hit at world distance g, TLAS nodes beyond g are skipped and
 //    the next instance is entered with the model-space bound t <= (g + |M o_m - o_w|) / |M3 d_m|.
+//  * ANY (ptap_query_occluded, DESIGN.md 4.8): every ray starts as if a winner at its segment length L = D[i].w existed, and retires
+//    as occluded at the first accepted triangle whose model's winner is provably nearer than L; the record it leaves otherwise is a
+//    closest-hit candidate that k_resolve_occluded compares with L.
 //
 // Node = 128 B = one L1 line: a node-local origin, four links, and four child boxes as binary32 offsets from that origin
 // (device_types.h: BvhNode); leaf-order triangle = 64 B with its global id (2 x LDG.E.256).  The node step costs one FMA per plane:
@@ -84,7 +87,7 @@ __device__ __forceinline__ void leafTriangle(const SceneDev& sc, const V3& o, co
 
 }  // namespace
 
-template <bool UV, bool COUNT>
+template <bool UV, bool COUNT, bool ANY = false>
 __global__ void __launch_bounds__(kTraceBlock, PTAP_TRACE_MIN_CTAS)
 k_trace_bvh(SceneDev sc, const float4* __restrict__ O, const float4* __restrict__ D, float4* __restrict__ hit,
             float2* __restrict__ uv, int4* __restrict__ counts, FrameState* st, int round, int n_fixed, unsigned long long* __restrict__ stamp)
@@ -151,6 +154,8 @@ k_trace_bvh(SceneDev sc, const float4* __restrict__ O, const float4* __restrict_
     int w_next = 0, w_end = 0;
     bool exhausted = false;
     const int vote_tri = sc.vote_tri, vote_inst = sc.vote_inst, vote_refill = sc.vote_refill;
+    // ANY only: the segment length L, the absolute slack cb of the exit step for this ray, world units per model-space t of the entered instance
+    float any_len = 0.0f, any_cb = 0.0f, any_scale = 0.0f;
 
     for (;;) {
         // ---- (1) inner nodes (TLAS and BLAS share the 4-wide format): test the four child boxes, continue with the nearest hit child,
@@ -201,10 +206,12 @@ k_trace_bvh(SceneDev sc, const float4* __restrict__ O, const float4* __restrict_
                 key[3] = childKey(nxb.y, nyb.y, nzb.y, fxb.y, fyb.y, fzb.y, tmin, tmax);
 #pragma unroll
                 for (int c = 0; c < 4; ++c) lnk[c] = __float_as_int(hd.v[4 + c]);
+                if (!ANY) {     // an any-hit traversal takes the hit children in node order: 3 % faster than nearest first (DESIGN 4.8)
 #define PTAP_CSWAP(a, b) { const bool sw = key[b] < key[a]; const int ka = sw ? key[b] : key[a], kb = sw ? key[a] : key[b]; \
                            const int la = sw ? lnk[b] : lnk[a], lb = sw ? lnk[a] : lnk[b]; key[a] = ka; key[b] = kb; lnk[a] = la; lnk[b] = lb; }
-                PTAP_CSWAP(0, 1) PTAP_CSWAP(2, 3) PTAP_CSWAP(0, 2) PTAP_CSWAP(1, 3) PTAP_CSWAP(1, 2)
+                    PTAP_CSWAP(0, 1) PTAP_CSWAP(2, 3) PTAP_CSWAP(0, 2) PTAP_CSWAP(1, 3) PTAP_CSWAP(1, 2)
 #undef PTAP_CSWAP
+                }
                 if (key[3] != 0x7f800000) push(lnk[3]);
                 if (key[2] != 0x7f800000) push(lnk[2]);
                 if (key[1] != 0x7f800000) push(lnk[1]);
@@ -223,7 +230,20 @@ k_trace_bvh(SceneDev sc, const float4* __restrict__ O, const float4* __restrict_
         // ---- (3a) one triangle of the held leaf (Renderer.cpp:174-215)
         if (s_tri && n_tri >= min(vote_tri, n_inner)) {
             leafTriangle<UV, COUNT>(sc, ro, rd, tmax, best_tri, best_u, best_v, (int)(code >> 3), cnt);
-            if (code & 7u) node = (int)~(code + 7u); else node = pop();   // (first + 1, count - 1), or pop when the leaf is finished
+            if constexpr (ANY) {
+                // The model's true winner has t in [-EPSILON, tmax] (the best accepted t so far), so its world distance is at most
+                // m = max(|tmax|, EPSILON) * ascale up to the exit step's slack m * tie + cb: when that is below L (at most kFloatMax), so
+                // is the closest hit.
+                bool occluded = false;
+                if (best_tri >= 0) {
+                    const float m = fmaxf(fabsf(tmax), kEpsilon) * any_scale;
+                    occluded = m + (m * sc.tie + any_cb) < any_len;
+                }
+                if (occluded) { sp = 0; node = kDone; g_model_f = __int_as_float(kAnyOccluded); }     // retire: empty stack, done state
+                else if (code & 7u) node = (int)~(code + 7u); else node = pop();
+            } else {
+                if (code & 7u) node = (int)~(code + 7u); else node = pop();   // (first + 1, count - 1), or pop when the leaf is finished
+            }
         }
         // ---- (3b) TLAS leaf: enter instance `im` (Renderer.cpp:381-384)
         if (s_enter && n_enter >= min(vote_inst, n_inner)) {
@@ -246,6 +266,7 @@ k_trace_bvh(SceneDev sc, const float4* __restrict__ O, const float4* __restrict_
                 const float tb = (g_dist * sc.prune + sc.c_pad + 1e-4f * (fabsf(bo.x) + fabsf(bo.y) + fabsf(bo.z))) * (mlen * wil) * 1.0001f;
                 if (tb < kFloatMax) tmax = tb;                                  // false for NaN / inf: no bound
             }
+            if constexpr (ANY) any_scale = __fdividef(1.0f, mlen * wil);      // the triangle step's copy of what is pushed next
             push(__float_as_int(__fdividef(1.0f, mlen * wil)));                  // world distance per unit of model-space t, for the exit step
             push((int)~(kExitBit | (unsigned)im));
             node = __float_as_int(__ldg(&inst->grid.z));                        // BLAS root of the instance's mesh
@@ -268,10 +289,11 @@ k_trace_bvh(SceneDev sc, const float4* __restrict__ O, const float4* __restrict_
                 bool take;
                 float nd = a;
                 if (a_hi < g_lo && a_hi < 0.99f * kFloatMax) take = true;        // clearly nearer than the current winner (or the first one)
-                else if (g_model >= 0 && a_lo > g_hi) take = false;              // clearly farther
+                else if ((ANY || g_model >= 0) && a_lo > g_hi) take = false;     // clearly farther (ANY: than L as well, so L keeps bounding)
                 else {                                                           // near-tie, or no usable bound: the reference's comparison
                     const float dn = exactHitDistance(sc, bo, bd, im, tmax);
-                    const float dg = g_model >= 0 ? exactHitDistance(sc, bo, bd, g_model, g_t) : kFloatMax;
+                    // ANY: a candidate must be nearer than the virtual winner at L (at kFloatMax when L is not below it) to be taken
+                    const float dg = g_model >= 0 ? exactHitDistance(sc, bo, bd, g_model, g_t) : ANY ? g_dist : kFloatMax;
                     take = dg > dn || (dg == dn && g_model >= 0 && im < g_model);   // Renderer.cpp:393 in model order
                     nd = dn;
                     if (!take && g_model >= 0) g_dist = dg;
@@ -292,7 +314,13 @@ k_trace_bvh(SceneDev sc, const float4* __restrict__ O, const float4* __restrict_
                 const bool found = g_dist < kFloatMax;
                 // hit.x < 0 (a constant: the consumers only test the sign) tells the consumer to evaluate the exact world distance
                 // from (model, t) (kernels.cuh: exactHitDistance)
-                hit[i] = make_float4(found ? -1.0f : kFloatMax, found ? g_tri_f : __int_as_float(-1), found ? g_model_f : __int_as_float(-1), g_t);
+                if constexpr (ANY) {
+                    // g_dist starts at L here, so a candidate is a taken model; model kAnyOccluded = retired early, -1 = no candidate
+                    const bool cand = __float_as_int(g_model_f) >= 0;
+                    hit[i] = make_float4(cand ? -1.0f : kFloatMax, cand ? g_tri_f : __int_as_float(-1), g_model_f, g_t);
+                } else {
+                    hit[i] = make_float4(found ? -1.0f : kFloatMax, found ? g_tri_f : __int_as_float(-1), found ? g_model_f : __int_as_float(-1), g_t);
+                }
                 if (UV && uv) uv[i] = make_float2(g_u, g_v);
                 if (COUNT) { if (counts) counts[i] = cnt; tot_x += cnt.x; tot_z += cnt.z; }
                 i = -1;
@@ -322,6 +350,14 @@ k_trace_bvh(SceneDev sc, const float4* __restrict__ O, const float4* __restrict_
                 if (COUNT) cnt = make_int4(0, 0, 0, 0);
                 sp = 0; push(kDone);
                 node = sc.tlas_root;
+                if constexpr (ANY) {
+                    // Hits at world distance >= kFloatMax are misses of the closest hit (the reference starts min_dist there), so
+                    // L >= kFloatMax (inf: "any hit") asks the same as L = kFloatMax; the comparison keeps NaN, which retires below.
+                    any_len = d4.w > kFloatMax ? kFloatMax : d4.w;
+                    any_cb = sc.c_pad + 1e-4f * (fabsf(bo.x) + fabsf(bo.y) + fabsf(bo.z));    // the exit step's cb for this ray
+                    if (any_len < kFloatMax) { g_dist = any_len; tmax = worldBound(any_len, sc.prune, any_cb); }   // a virtual winner at L
+                    if (!(any_len > 0.0f)) node = pop();                         // L <= 0 or NaN: nothing can be nearer; retire (kDone)
+                }
             }
             w_next += min(__popc(m_done), avail);
         }
@@ -345,6 +381,11 @@ k_trace_bvh(SceneDev sc, const float4* __restrict__ O, const float4* __restrict_
 #undef g_tri_f
 #undef g_u
 #undef g_v
+
+void launchTraceBvhAny(const SceneDev& sc, const float4* O, const float4* D, float4* hit, FrameState* st, int n, int grid, cudaStream_t stream)
+{
+    k_trace_bvh<false, false, true><<<grid, kTraceBlock, 0, stream>>>(sc, O, D, hit, nullptr, nullptr, st, 0, n, nullptr);
+}
 
 void launchTraceBvh(const SceneDev& sc, const float4* O, const float4* D, float4* hit, float2* uv, int4* counts, bool count_totals,
                      FrameState* st, int round, int n_fixed, int grid, cudaStream_t stream, unsigned long long* stamp)

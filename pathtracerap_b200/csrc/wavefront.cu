@@ -374,6 +374,24 @@ __global__ void k_resolve_hits(SceneDev sc, const float4* __restrict__ O, const 
     out[i] = r;
 }
 
+// occlusion of a segment of world length L = D[i].w (ptap_query_occluded): the closest hit is nearer than L.  A record is a closest hit
+// (launchTrace), or what the any-hit traversal left: retired as occluded (model kAnyOccluded), a candidate (model, t) to compare, or a miss.
+__global__ void k_resolve_occluded(SceneDev sc, const float4* __restrict__ O, const float4* __restrict__ D, const float4* __restrict__ hit,
+                                   int n, uint8_t* __restrict__ occluded)
+{
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const float4 h = hit[i];
+    const int model = __float_as_int(h.z);
+    bool occ = model == kAnyOccluded;
+    if (h.x < kFloatMax && model >= 0) {
+        const float4 d4 = D[i];
+        const float dist = h.x >= 0.0f ? h.x : exactHitDistance(sc, v3(O[i]), v3(d4), model, h.w);   // as k_resolve_hits
+        occ = dist < d4.w;                                                                      // NaN L: false
+    }
+    occluded[i] = occ ? 1 : 0;
+}
+
 __global__ void k_set_iter(FrameState* st, int iter) { st->iter_next = iter; }
 
 // normals[t] = flat normal of global triangle t (the .w lanes of its TriRec), one 16-byte record for the shade kernel's gather
@@ -449,6 +467,11 @@ int shadeOccupancy()
 void launchResolveHits(const SceneDev& sc, const float4* O, const float4* D, const float4* hit, const float2* uv, int n, PtapHit* out, cudaStream_t stream)
 {
     if (n > 0) k_resolve_hits<<<(n + 255) / 256, 256, 0, stream>>>(sc, O, D, hit, uv, n, out);
+}
+
+void launchResolveOccluded(const SceneDev& sc, const float4* O, const float4* D, const float4* hit, int n, uint8_t* occluded, cudaStream_t stream)
+{
+    if (n > 0) k_resolve_occluded<<<(n + 255) / 256, 256, 0, stream>>>(sc, O, D, hit, n, occluded);
 }
 
 void launchSetIter(FrameState* st, int iter, cudaStream_t stream) { k_set_iter<<<1, 1, 0, stream>>>(st, iter); }

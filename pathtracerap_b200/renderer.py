@@ -6,6 +6,7 @@ methods expose what the reference hard-codes (resolution, iterations, depth) and
 from __future__ import annotations
 
 import ctypes as C
+import numbers
 
 import numpy as np
 
@@ -20,6 +21,7 @@ class Renderer:
     def __init__(self, device: int = 0, width: int | None = None, height: int | None = None, iters: int | None = None,
                  depth: int | None = None, accel: int = N.ACCEL_GRID_EMULATED, first_hit_cache: bool = True, profile: bool = False,
                  arena_bytes: int = 0):
+        self.device = device
         self.W = width or self.RESOLUTION_X; self.H = height or self.RESOLUTION_Y
         self.iters = iters or self.ITER; self.depth = depth or self.DEPTH
         self.accel = accel
@@ -184,6 +186,81 @@ class Renderer:
         d = {k: getattr(s, k) for k, _ in N.Stats._fields_ if k != "active_per_round"}
         d["active_per_round"] = [int(x) for x in s.active_per_round]
         return d
+
+    # -- ray queries on device tensors (ptap.h: ptap_query_closest / ptap_query_occluded) -----------------------------------------
+    def _check_rays(self, org, dir):
+        import torch
+        for name, x in (("org", org), ("dir", dir)):
+            if not isinstance(x, torch.Tensor):
+                raise TypeError(f"{name} must be a torch tensor, got {type(x).__name__}")
+            if x.dtype != torch.float32:
+                raise TypeError(f"{name} must be float32, got {x.dtype}")
+            if x.device.type != "cuda":
+                raise ValueError(f"{name} is on {x.device}: the queries read device memory")
+            if x.device.index != self.device:
+                raise ValueError(f"{name} is on {x.device}, the renderer on cuda:{self.device}")
+            if x.dim() != 2 or x.shape[1] not in (3, 4):
+                raise ValueError(f"{name} must have shape (n, 3) or (n, 4), got {tuple(x.shape)}")
+            if not x.is_contiguous():
+                raise ValueError(f"{name} must be contiguous")
+        if org.shape[0] != dir.shape[0]:
+            raise ValueError(f"org has {org.shape[0]} rays, dir {dir.shape[0]}")
+
+    @staticmethod
+    def _pack_rays(org, dir, length=None):
+        """(n, 4) float32 origins and directions in the ABI's layout, dir[:, 3] = length when given (a copy only where needed)."""
+        import torch
+        n = org.shape[0]
+        o4 = org if org.shape[1] == 4 else torch.cat([org, org.new_zeros((n, 1))], dim=1)
+        if length is None:
+            d4 = dir if dir.shape[1] == 4 else torch.cat([dir, dir.new_zeros((n, 1))], dim=1)
+        else:
+            d4 = torch.empty((n, 4), dtype=torch.float32, device=dir.device)
+            d4[:, :3] = dir[:, :3]
+            d4[:, 3] = length
+        return o4, d4
+
+    def _stream_handle(self):
+        import torch
+        # torch's default stream is the legacy NULL stream: name it (cudaStreamLegacy) so that the query is ordered with it, since NULL
+        # would mean the renderer's own stream
+        return torch.cuda.current_stream(self.device).cuda_stream or 1
+
+    def query_closest(self, org, dir) -> dict:
+        """Closest hit of every ray (o, d) of two (n, 3) or (n, 4) float32 CUDA tensors, on the current torch stream, without a host
+        synchronisation: what trace() returns for the same rays, bit for bit.  A dict of views of one (n, 10) int32 tensor holding the
+        PtapHit records: model, tri, t_model, dist, u, v, normal (n, 3), mat_type (model = -1: miss)."""
+        import torch
+        self._check_rays(org, dir)
+        o4, d4 = self._pack_rays(org, dir)
+        n = o4.shape[0]
+        rec = torch.empty((n, 10), dtype=torch.int32, device=o4.device)
+        self._check(N.lib().ptap_query_closest(self.h, o4.data_ptr(), d4.data_ptr(), n, rec.data_ptr(), self._stream_handle()), "query_closest")
+        f = rec.view(torch.float32)
+        return {"model": rec[:, 0], "tri": rec[:, 1], "t_model": f[:, 2], "dist": f[:, 3], "u": f[:, 4], "v": f[:, 5],
+                "normal": f[:, 6:9], "mat_type": rec[:, 9]}
+
+    def query_occluded(self, org, dir, tmax):
+        """Is the segment from o along d of world length tmax blocked: closest.model >= 0 and closest.dist < tmax (binary32; inf = any
+        hit, NaN = False).  tmax is a float or an (n,) float32 tensor on the same device.  A torch.bool tensor (n,), on the current stream."""
+        import torch
+        self._check_rays(org, dir)
+        if isinstance(tmax, torch.Tensor):
+            if tmax.dtype != torch.float32:
+                raise TypeError(f"tmax must be float32, got {tmax.dtype}")
+            if tmax.device != org.device:
+                raise ValueError(f"tmax is on {tmax.device}, the rays on {org.device}")
+            if tuple(tmax.shape) != (org.shape[0],):
+                raise ValueError(f"tmax must have shape ({org.shape[0]},), got {tuple(tmax.shape)}")
+        elif isinstance(tmax, numbers.Real) and not isinstance(tmax, (bool, np.bool_)):      # Python and numpy scalars
+            tmax = float(tmax)
+        else:
+            raise TypeError(f"tmax must be a float or a tensor, got {type(tmax).__name__}")
+        o4, d4 = self._pack_rays(org, dir, tmax)
+        n = o4.shape[0]
+        out = torch.empty(n, dtype=torch.bool, device=o4.device)
+        self._check(N.lib().ptap_query_occluded(self.h, o4.data_ptr(), d4.data_ptr(), n, out.data_ptr(), self._stream_handle()), "query_occluded")
+        return out
 
     # -- parity entry points -------------------------------------------------------------------------------------
     def trace(self, rays_od, counts: bool = False):
