@@ -350,6 +350,17 @@ int buildTlas(std::vector<TlasItem>& items, int b, int e, std::vector<Bvh2Node>&
     return me;
 }
 
+// Both builders write the scene arena's nodes in place: from then on the tree that was there is gone, and until the new one is complete
+// (finishBvh) there is none to trace.  A build that fails - a tree too deep for the traversal stack, say - leaves the context without a
+// BVH, and every entry point that would traverse one refuses (bvhMissing).
+void dropBvh(ptap_ctx* ctx)
+{
+    ctx->have_bvh = false; ctx->bvh_kind = -1; ctx->sc.tlas_root = -1;
+}
+
+// The BVH modes and the emulated grid walk traverse the BVH.
+bool bvhMissing(const ptap_ctx* ctx) { return ctx->accel != PTAP_ACCEL_GRID_COMPAT && !ctx->have_bvh; }
+
 // Second half of every BVH build: points every model at its mesh's root, derives the instances' world boxes from the BLAS root bounds
 // (`roots[m]` = host copy of mesh m's root node), builds the TLAS over them behind the `nnodes` BLAS nodes and publishes the scene fields.
 int finishBvh(ptap_ctx* ctx, const BvhNode* roots, const int* mesh_root, int nnodes, int blas_depth, size_t* tlas_bytes)
@@ -439,6 +450,7 @@ int finishBvh(ptap_ctx* ctx, const BvhNode* roots, const int* mesh_root, int nno
 int uploadBvh(ptap_ctx* ctx, const BvhNode* nodes, int nnodes, const int* tri_id, const int* mesh_root, int known_depth, size_t* bytes)
 {
     const int nt = ctx->ntris, nm = (int)ctx->h_models.size();
+    dropBvh(ctx);
     if ((size_t)nnodes > ctx->nodes_cap) return fail(ctx, PTAP_E_NOMEM, "BVH has more nodes than reserved (2 per triangle)");
     // range checks of every link and leaf-order entry: 90 MB of host memory for a 1.3 M-triangle scene, on every upload - spread over threads
     {
@@ -516,6 +528,7 @@ int uploadBvh(ptap_ctx* ctx, const BvhNode* nodes, int nnodes, const int* tri_id
 int buildBvhOnDevice(ptap_ctx* ctx)
 {
     const int nt = ctx->ntris, nmesh = (int)ctx->h_meshes.size();
+    dropBvh(ctx);
     int max_tris = 0;
     for (const PtapMesh& m : ctx->h_meshes) max_tris = std::max(max_tris, m.t_end - m.t_start);
     const size_t need = deviceBvhScratchBytes(max_tris);
@@ -528,9 +541,10 @@ int buildBvhOnDevice(ptap_ctx* ctx)
         if (n <= 0 || m.t_start < 0 || m.t_end > nt) continue;
         if ((size_t)nnodes + (size_t)n > ctx->nodes_cap || leaf_base + n > nt) return fail(ctx, PTAP_E_NOMEM, "device BVH build: node / leaf storage exhausted");
         int made = 0, depth = 0;
+        std::string why;
         const int e = buildMeshBvhDevice(ctx->d_tris, m.t_start, m.t_end, m.bb_min, m.bb_max, nnodes, ctx->d_nodes + nnodes, leaf_base, ctx->d_btris, ctx->d_btid,
-                                         ctx->scratch.base, ctx->scratch.cap, ctx->stream, &made, &depth);
-        if (e != 0) return fail(ctx, e, "device BVH build of mesh %d: %s", mi, cudaGetErrorString((cudaError_t)e));
+                                         ctx->scratch.base, ctx->scratch.cap, ctx->stream, &made, &depth, &why);
+        if (e != 0) return fail(ctx, e, "device BVH build of mesh %d (%d triangles): %s", mi, n, why.empty() ? cudaGetErrorString((cudaError_t)e) : why.c_str());
         mesh_root[mi] = nnodes;
         nnodes += made; leaf_base += n; blas_depth = std::max(blas_depth, depth);
     }
@@ -914,6 +928,7 @@ int ptap_render(ptap_ctx* ctx, int32_t iter_begin, int32_t iter_end)
 {
     if (!ctx || !ctx->have_scene || !ctx->have_frame) return fail(ctx, PTAP_E_STATE, "render: scene and render parameters required");
     if ((ctx->accel == PTAP_ACCEL_GRID_COMPAT || ctx->accel == PTAP_ACCEL_GRID_EMULATED) && !ctx->have_grid) return fail(ctx, PTAP_E_STATE, "render: no grid in the uploaded scene; build the BVH");
+    if (bvhMissing(ctx)) return fail(ctx, PTAP_E_STATE, "render: no BVH on the device (build_accel failed or was not called)");
     if (iter_end < iter_begin) return fail(ctx, PTAP_E_INVALID, "render: empty iteration range");
     CK(cudaSetDevice(ctx->device));
     if (ctx->render_pending) { int rc = collect(ctx); if (rc) return rc; }
@@ -1156,6 +1171,7 @@ static int traceImpl(ptap_ctx* ctx, const float* rays_od, int32_t n, PtapHit* ou
 {
     if (!ctx || !ctx->have_scene || !rays_od || !out || n < 0) return fail(ctx, PTAP_E_STATE, "trace: scene and buffers required");
     if ((ctx->accel == PTAP_ACCEL_GRID_COMPAT || ctx->accel == PTAP_ACCEL_GRID_EMULATED) && !ctx->have_grid) return fail(ctx, PTAP_E_STATE, "trace: no grid in the uploaded scene");
+    if (bvhMissing(ctx)) return fail(ctx, PTAP_E_STATE, "trace: no BVH on the device (build_accel failed or was not called)");
     if (n == 0) return PTAP_OK;
     CK(cudaSetDevice(ctx->device));
     if (ctx->render_pending) { int rc = collect(ctx); if (rc) return rc; }
@@ -1214,6 +1230,7 @@ static int queryImpl(ptap_ctx* ctx, const char* call, const float* org, const fl
     if (n == 0) return PTAP_OK;
     if (!ctx->have_scene) return fail(ctx, PTAP_E_STATE, "%s: no scene uploaded", call);
     if ((ctx->accel == PTAP_ACCEL_GRID_COMPAT || ctx->accel == PTAP_ACCEL_GRID_EMULATED) && !ctx->have_grid) return fail(ctx, PTAP_E_STATE, "%s: no grid in the uploaded scene", call);
+    if (bvhMissing(ctx)) return fail(ctx, PTAP_E_STATE, "%s: no BVH on the device (build_accel failed or was not called)", call);
     CK(cudaSetDevice(ctx->device));
     { const int rc = checkQueryPtr(ctx, call, "org", org, 16); if (rc) return rc; }
     { const int rc = checkQueryPtr(ctx, call, "dir", dir, 16); if (rc) return rc; }
@@ -1344,6 +1361,7 @@ int ptap_shade(ptap_ctx* ctx, const PtapPathIn* paths, int32_t n, int32_t iter, 
 int ptap_bench_trace(ptap_ctx* ctx, const float* rays_od, int32_t n, int32_t reps, float* ms_per_launch)
 {
     if (!ctx || !ctx->have_scene || !rays_od || n <= 0 || reps <= 0 || !ms_per_launch) return fail(ctx, PTAP_E_INVALID, "bench_trace: bad arguments");
+    if (bvhMissing(ctx)) return fail(ctx, PTAP_E_STATE, "bench_trace: no BVH on the device (build_accel failed or was not called)");
     CK(cudaSetDevice(ctx->device));
     if (ctx->render_pending) { int rc = collect(ctx); if (rc) return rc; }
     size_t need = Arena::need(n, sizeof(float4)) * 3 + Arena::need(1, sizeof(FrameState)) + (ctx->accel == PTAP_ACCEL_GRID_EMULATED ? emuArenaNeed(ctx, n) : 0) + 4096;
@@ -1383,6 +1401,7 @@ int ptap_render_probe(ptap_ctx* ctx, int32_t iter, int32_t round, float* rays_od
 {
     if (!ctx || !ctx->have_scene || !ctx->have_frame) return fail(ctx, PTAP_E_STATE, "render_probe: scene and render parameters required");
     if ((ctx->accel == PTAP_ACCEL_GRID_COMPAT || ctx->accel == PTAP_ACCEL_GRID_EMULATED) && !ctx->have_grid) return fail(ctx, PTAP_E_STATE, "render_probe: no grid in the uploaded scene");
+    if (bvhMissing(ctx)) return fail(ctx, PTAP_E_STATE, "render_probe: no BVH on the device (build_accel failed or was not called)");
     if (round < 0 || round >= ctx->wv.depth || !n_out || cap < 0) return fail(ctx, PTAP_E_INVALID, "render_probe: bad arguments");
     CK(cudaSetDevice(ctx->device));
     if (ctx->render_pending) { int rc = collect(ctx); if (rc) return rc; }

@@ -286,18 +286,28 @@ __global__ void k_ploc_init(const Box6* __restrict__ leaf_box, int n, Box6* __re
     if (i < n) { cbox[i] = leaf_box[i]; cnode[i] = ~i; }
 }
 
-// nearest[i] = the position within the radius whose union with cluster i has the smallest area (ties: the lower position)
+// Tie key of the pair {i, j}, the same from either end: the partner in the same aligned pair (i >> 1 == j >> 1) first, then the nearer
+// position, then the lower one.  A rule that is not symmetric (such as "the lower position") lets tied clusters point along a chain, i -> i - 1,
+// in which only the first pair is mutual: coincident triangles or a long ribbon of equal quads then merge one pair per round.
+__device__ __forceinline__ unsigned long long plocTieKey(int i, int j)
+{
+    return ((unsigned long long)((i >> 1) != (j >> 1)) << 63) | ((unsigned long long)abs(i - j) << 32) | (unsigned)min(i, j);
+}
+
+// nearest[i] = the position within the radius whose union with cluster i has the smallest area, ties broken by plocTieKey.  The order on
+// (area, key) is the same for both ends of every pair, so the globally smallest pair is mutual and every round merges.
 __global__ void k_ploc_nearest(const Box6* __restrict__ cbox, int n, int* __restrict__ nearest)
 {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     const Box6 me = cbox[i];
-    float best = 3e38f; int bj = -1;
+    float best = 3e38f; int bj = -1; unsigned long long bkey = ~0ull;
     const int j0 = max(0, i - kPlocRadius), j1 = min(n - 1, i + kPlocRadius);
     for (int j = j0; j <= j1; ++j) {
         if (j == i) continue;
         const float a = unionArea(me, cbox[j]);
-        if (a < best) { best = a; bj = j; }
+        const unsigned long long key = plocTieKey(i, j);
+        if (a < best || (a == best && key < bkey)) { best = a; bj = j; bkey = key; }
     }
     nearest[i] = bj;
 }
@@ -404,9 +414,10 @@ size_t deviceBvhScratchBytes(int ntris)
 }
 
 // Builds the BLAS of one mesh (triangles [t0, t1) of the global table) into out_nodes[0 .. *nnodes) with links relative to node_base,
-// leaf-order triangles into btris / btid at [leaf_base, leaf_base + n).  Returns a cudaError_t; *depth = levels of 4-wide nodes.
+// leaf-order triangles into btris / btid at [leaf_base, leaf_base + n).  Returns a cudaError_t; *depth = levels of 4-wide nodes.  When the
+// build itself gives up (not a CUDA call), *why says why.
 int buildMeshBvhDevice(const TriRec* d_tris, int t0, int t1, const float* bb_min, const float* bb_max, int node_base, BvhNode* out_nodes, int leaf_base,
-                       LeafTri* btris, int* btid, char* scratch, size_t scratch_bytes, cudaStream_t stream, int* nnodes, int* depth)
+                       LeafTri* btris, int* btid, char* scratch, size_t scratch_bytes, cudaStream_t stream, int* nnodes, int* depth, std::string* why)
 {
     const int n = t1 - t0, L = (n + kCluster - 1) / kCluster;
     *nnodes = 0; *depth = 0;
@@ -476,7 +487,10 @@ int buildMeshBvhDevice(const TriRec* d_tris, int t0, int t1, const float* bb_min
             if (e == cudaSuccess) e = cudaStreamSynchronize(stream);
             if (e != cudaSuccess) return e;
             const int m2 = last[0] + last[1];
-            if (m2 >= m || ++rounds > 4096) return cudaErrorUnknown;      // every round merges at least the globally best pair
+            if (m2 >= m || ++rounds > 4096) {                              // every round merges at least the globally best pair
+                if (why) *why = "PLOC merging stalled at " + std::to_string(m2) + " of " + std::to_string(L) + " clusters after " + std::to_string(rounds) + " rounds";
+                return cudaErrorUnknown;
+            }
             m = m2;
             std::swap(cb, cb2); std::swap(cn, cn2);
         }
@@ -528,7 +542,7 @@ int buildMeshBvhDevice(const TriRec* d_tris, int t0, int t1, const float* bb_min
         e = cudaMemcpyAsync(counters + 1, &zero, sizeof zero, cudaMemcpyHostToDevice, stream);
         if (e != cudaSuccess) return e;
         std::swap(cur, nxt);
-        if (levels > 200) return cudaErrorUnknown;
+        if (levels > 200) { if (why) *why = "the 4-wide collapse exceeded 200 levels"; return cudaErrorUnknown; }
     }
     *depth = levels;
     return cudaGetLastError();

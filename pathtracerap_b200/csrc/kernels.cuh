@@ -1,5 +1,7 @@
 // kernels.cuh - launch wrappers of the wavefront kernels (one translation unit per kernel family).
 #pragma once
+#include <string>
+
 #include "device_types.h"
 #include "exact_math.cuh"
 #include "../../include/ptap.h"
@@ -67,7 +69,8 @@ void launchTraceBvhAny(const SceneDev& sc, const float4* O, const float4* D, flo
 // bvh_device.cu
 size_t deviceBvhScratchBytes(int ntris);
 int buildMeshBvhDevice(const TriRec* d_tris, int t0, int t1, const float* bb_min, const float* bb_max, int node_base, BvhNode* out_nodes, int leaf_base,
-                       LeafTri* btris, int* btid, char* scratch, size_t scratch_bytes, cudaStream_t stream, int* nnodes, int* depth);
+                       LeafTri* btris, int* btid, char* scratch, size_t scratch_bytes, cudaStream_t stream, int* nnodes, int* depth,
+                       std::string* why);
 
 // grid_device.cu: Scene::addMeshesToGrid on the device, one mesh's grid at a time
 int gridDeviceCount(const float* d_pos, int t0, int n, const float bb_min[3], const float width[3], const int gd[3], int* d_count, int* d_offset,
