@@ -34,8 +34,9 @@
 extern "C" {
 #endif
 
-#define PTAP_VERSION 3      /* 2: PtapBvhNode carries node-local offsets; ptap_render_probe, ptap_reduce*, stamps
-                               3: ray queries on device buffers, ptap_query_closest / ptap_query_occluded */
+#define PTAP_VERSION 4      /* 2: PtapBvhNode carries node-local offsets; ptap_render_probe, ptap_reduce*, stamps
+                               3: ray queries on device buffers, ptap_query_closest / ptap_query_occluded
+                               4: ptap_update_models */
 
 enum {
     PTAP_OK = 0,
@@ -221,6 +222,16 @@ const char* ptap_last_error(const ptap_ctx* ctx);
 /* Renderer::allocateOnGPU (Renderer.cpp:65-130): copies the scene into the device arena (repacked, see DESIGN.md). */
 int ptap_upload_scene(ptap_ctx* ctx, const PtapSceneView* view);
 int ptap_build_accel(ptap_ctx* ctx, int kind);
+/* Replace the records of models [first, first + count) of the uploaded scene: transforms and material.  mesh_index and grid_index must
+ * equal the uploaded ones (anything else needs ptap_upload_scene).  The instance records and, when a BVH is on the device, the TLAS are
+ * rebuilt on the GPU; BLAS, triangles and grids are untouched.  Ordered after everything already enqueued on ptap_stream(ctx); returns when
+ * the device work is done.  Afterwards every entry point behaves exactly as after ptap_upload_scene + ptap_build_accel(current accel) of
+ * the scene with these models: hits, films and query answers bit for bit (the TLAS is a different tree, so traversal counts and
+ * PTAP_FLAG_COUNT averages may differ).  The first-hit cache is forgotten.  count == 0 is a no-op.
+ * Errors: PTAP_E_STATE without an uploaded scene; PTAP_E_INVALID for a bad range, a changed mesh_index or grid_index or a singular
+ * world_to_model, checked before anything changes (the context then traces exactly as before the call).  A failure after these checks (a
+ * CUDA error, a TLAS too deep for the traversal stack) keeps the new models but drops the BVH: ptap_build_accel builds it again. */
+int ptap_update_models(ptap_ctx* ctx, const PtapModel* models, int32_t first, int32_t count);
 /* Scene::addMeshesToGrid (Scene.cpp:318-396) on the DEVICE for the scene last uploaded (`view` must be that scene's view: vertices and
  * triangles are read again): one gx x gy x gz grid per distinct mesh in model order, built by sorting (cell, triangle) pairs; cells and
  * reference lists are bit-identical to the host builder's / the reference's (ascending triangle order per cell).  Selects

@@ -70,7 +70,7 @@ EXPORTS = [
     "ptap_create", "ptap_destroy", "ptap_last_error", "ptap_upload_scene", "ptap_build_accel", "ptap_build_grids_device", "ptap_read_grids", "ptap_set_render_params",
     "ptap_render", "ptap_timer_start", "ptap_timer_stop", "ptap_frame_begin", "ptap_film_reset", "ptap_sync", "ptap_read_film", "ptap_film_device_ptr", "ptap_film_add",
     "ptap_write_bmp", "ptap_read_film_resolved", "ptap_write_bmp_resolved", "ptap_get_stats", "ptap_stream", "ptap_trace", "ptap_trace_count", "ptap_shade", "ptap_bench_trace", "ptap_render_probe", "ptap_get_iteration_times",
-    "ptap_query_closest", "ptap_query_occluded",
+    "ptap_query_closest", "ptap_query_occluded", "ptap_update_models",
     "ptap_reduce_peer", "ptap_nccl_unique_id", "ptap_nccl_init", "ptap_reduce", "ptap_nccl_finalize",
 ]
 
@@ -140,6 +140,7 @@ def lib():
         L.ptap_get_iteration_times.argtypes = [vp, vp, ci, C.POINTER(ci)]
         L.ptap_query_closest.argtypes = [vp, vp, vp, ci, vp, vp]
         L.ptap_query_occluded.argtypes = [vp, vp, vp, ci, vp, vp]
+        L.ptap_update_models.argtypes = [vp, vp, ci, ci]
         L.ptap_reduce_peer.argtypes = [vp, vp]
         L.ptap_nccl_unique_id.argtypes = [vp]
         L.ptap_nccl_init.argtypes = [vp, vp, ci, ci]

@@ -153,12 +153,6 @@ void encodeNode(BvhNode& nd, const ChildBox boxes[4], unsigned used)
         }
 }
 
-void decodeChild(const BvhNode& nd, int c, double lo[3], double hi[3])
-{
-    const double p[3] = {nd.px, nd.py, nd.pz};
-    for (int k = 0; k < 3; ++k) { lo[k] = p[k] + (double)nd.planes[k][0][c]; hi[k] = p[k] + (double)nd.planes[k][1][c]; }
-}
-
 long long validateBvh(const BvhNode* nodes, int nnodes, int root, int nleafprims, const std::function<ChildBox(int)>& prim_box, int* depth)
 {
     // A ray that must reach a primitive has to enter EVERY child box on the path from the root, so each primitive's box is checked against

@@ -20,9 +20,13 @@ struct ChildBox { float lo[3], hi[3]; };
 // Fills the boxes of node `nd` from up to four (slot, box) pairs: local origin, binary32 offsets rounded outward after a margin that
 // covers the traversal's own arithmetic; unused slots get an inverted box.  `boxes[c]` is read only when bit c of `used` is set.
 void encodeNode(BvhNode& nd, const ChildBox boxes[4], unsigned used);
-// Decoded box of slot c (what the traversal kernel tests), in double: p + offset.
-void decodeChild(const BvhNode& nd, int c, double lo[3], double hi[3]);
-inline bool slotUsed(const BvhNode& nd, int c) { return nd.planes[0][0][c] <= nd.planes[0][1][c]; }
+// Decoded box of slot c (what the traversal kernel tests), in double: p + offset.  Host and device (instance_math.h).
+__host__ __device__ inline void decodeChild(const BvhNode& nd, int c, double lo[3], double hi[3])
+{
+    const double p[3] = {nd.px, nd.py, nd.pz};
+    for (int k = 0; k < 3; ++k) { lo[k] = p[k] + (double)nd.planes[k][0][c]; hi[k] = p[k] + (double)nd.planes[k][1][c]; }
+}
+__host__ __device__ inline bool slotUsed(const BvhNode& nd, int c) { return nd.planes[0][0][c] <= nd.planes[0][1][c]; }
 
 // Collapses the binary subtree rooted at node `root2` of `n2` into 4-wide nodes appended to `out` (absolute index = base + position in
 // `out`): a child is replaced by its own two children, largest box first, until the node has four.  Returns the new root's index.

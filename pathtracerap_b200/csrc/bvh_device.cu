@@ -20,7 +20,9 @@
 // The tree is a different one than the host builder's, so rays visit different boxes; hits are bit-identical all the same, because the
 // boxes are conservative for the reference's predicate and the triangle arithmetic is the exact one (tests/test_gpu_device_bvh.py).
 #include <algorithm>
+#include <climits>
 #include <cmath>
+#include <cstring>
 #include <cstdlib>
 #include <string>
 #include <utility>
@@ -29,6 +31,8 @@
 #include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_scan.cuh>
 
+#include "host_math.h"
+#include "instance_math.h"
 #include "kernels.cuh"
 
 namespace ptap {
@@ -208,10 +212,15 @@ __device__ void encodeNodeDevice(BvhNode& nd, const Box6* boxes, int ne)
         }
 }
 
-// One breadth-first level: frontier item = (binary internal node, index of the 4-wide node that represents it).
+// Leaf c of a TLAS (INST): instance leaf ~(0x20000000 | model), the model being leaf_model[c]
+__device__ __forceinline__ int instLeafLink(const int* __restrict__ leaf_model, int c) { return ~(0x20000000 | leaf_model[c]); }
+
+// One breadth-first level: frontier item = (binary internal node, index of the 4-wide node that represents it).  INST: the leaves are
+// instances (a TLAS, leaf_model), else triangle clusters.
+template <bool INST = false>
 __global__ void k_lbvh_collapse(const int2* __restrict__ child, const Box6* __restrict__ node_box, const Box6* __restrict__ leaf_box, int n, int leaf_base,
                                 const int2* __restrict__ frontier, int nfrontier, int2* __restrict__ next, int* __restrict__ counters /* [0] nodes, [1] next size */,
-                                int node_base, BvhNode* __restrict__ out)
+                                int node_base, BvhNode* __restrict__ out, const int* __restrict__ leaf_model = nullptr)
 {
     const int f = blockIdx.x * blockDim.x + threadIdx.x;
     if (f >= nfrontier) return;
@@ -246,19 +255,20 @@ __global__ void k_lbvh_collapse(const int2* __restrict__ child, const Box6* __re
                 const int idx = atomicAdd(&counters[0], 1);
                 next[atomicAdd(&counters[1], 1)] = make_int2(e, idx);
                 nd.link[k] = node_base + idx;
-            } else nd.link[k] = leafLink(~e, n, leaf_base);
+            } else nd.link[k] = INST ? instLeafLink(leaf_model, ~e) : leafLink(~e, n, leaf_base);
         } else nd.link[k] = nd.link[0];
     }
     encodeNodeDevice(nd, boxes, ne);
     out[item.y] = nd;
 }
 
-// a mesh whose triangles fit one leaf: a root with a single child
-__global__ void k_lbvh_single(const Box6* __restrict__ leaf_box, int n, int leaf_base, BvhNode* __restrict__ out)
+// a mesh whose triangles fit one leaf (a scene with one instance): a root with a single child
+template <bool INST = false>
+__global__ void k_lbvh_single(const Box6* __restrict__ leaf_box, int n, int leaf_base, BvhNode* __restrict__ out, const int* __restrict__ leaf_model = nullptr)
 {
     BvhNode nd;
     const Box6 b = leaf_box[0];
-    for (int k = 0; k < 4; ++k) nd.link[k] = leafLink(0, n, leaf_base);
+    for (int k = 0; k < 4; ++k) nd.link[k] = INST ? instLeafLink(leaf_model, 0) : leafLink(0, n, leaf_base);
     encodeNodeDevice(nd, &b, 1);
     out[0] = nd;
 }
@@ -399,78 +409,81 @@ template <typename T> T* carve(char*& p, size_t count)
     return r;
 }
 
-}  // namespace
-
-size_t deviceBvhScratchBytes(int ntris)
+size_t cubBytes(int n, int end_bit)
 {
-    const size_t n = (size_t)std::max(ntris, 1), L = (n + kCluster - 1) / kCluster;
-    size_t cub_bytes = 0;
-    cub::DeviceRadixSort::SortPairs(nullptr, cub_bytes, (const unsigned*)nullptr, (unsigned*)nullptr, (const int*)nullptr, (int*)nullptr, (int)n, 0, 30);
-    size_t scan_bytes = 0;
-    cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, (const int*)nullptr, (int*)nullptr, (int)n);
-    cub_bytes = std::max(cub_bytes, scan_bytes);
-    return 4 * ((n * 4 + 255) & ~size_t(255)) + cub_bytes + 256 + 4 * ((L * sizeof(Box6) + 255) & ~size_t(255)) + ((L * 8 + 255) & ~size_t(255)) * 4 +
+    size_t sort_bytes = 0, scan_bytes = 0;
+    cub::DeviceRadixSort::SortPairs(nullptr, sort_bytes, (const unsigned*)nullptr, (unsigned*)nullptr, (const int*)nullptr, (int*)nullptr, n, 0, end_bit);
+    cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, (const int*)nullptr, (int*)nullptr, n);
+    return std::max(sort_bytes, scan_bytes);
+}
+
+// carveBuild's bytes for `count` primitives in `leaves` leaves
+size_t scratchBytes(int count, int leaves, int end_bit)
+{
+    const size_t n = (size_t)std::max(count, 1), L = (size_t)std::max(leaves, 1);
+    return 4 * ((n * 4 + 255) & ~size_t(255)) + cubBytes((int)n, end_bit) + 256 + 4 * ((L * sizeof(Box6) + 255) & ~size_t(255)) + ((L * 8 + 255) & ~size_t(255)) * 4 +
            ((L * 4 + 255) & ~size_t(255)) * 3 + 4096;
 }
 
-// Builds the BLAS of one mesh (triangles [t0, t1) of the global table) into out_nodes[0 .. *nnodes) with links relative to node_base,
-// leaf-order triangles into btris / btid at [leaf_base, leaf_base + n).  Returns a cudaError_t; *depth = levels of 4-wide nodes.  When the
-// build itself gives up (not a CUDA call), *why says why.
-int buildMeshBvhDevice(const TriRec* d_tris, int t0, int t1, const float* bb_min, const float* bb_max, int node_base, BvhNode* out_nodes, int leaf_base,
-                       LeafTri* btris, int* btid, char* scratch, size_t scratch_bytes, cudaStream_t stream, int* nnodes, int* depth, std::string* why)
-{
-    const int n = t1 - t0, L = (n + kCluster - 1) / kCluster;
-    *nnodes = 0; *depth = 0;
-    if (n <= 0) return cudaSuccess;
-    if (deviceBvhScratchBytes(n) > scratch_bytes) return cudaErrorMemoryAllocation;
-    char* p = scratch;
-    unsigned* keys = carve<unsigned>(p, n); unsigned* keys2 = carve<unsigned>(p, n);
-    int* ids = carve<int>(p, n); int* ids2 = carve<int>(p, n);
-    size_t cub_bytes = 0;
-    cub::DeviceRadixSort::SortPairs(nullptr, cub_bytes, (const unsigned*)keys, keys2, (const int*)ids, ids2, n, 0, 30);
-    { size_t scan_bytes = 0; cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, (const int*)nullptr, (int*)nullptr, n); cub_bytes = std::max(cub_bytes, scan_bytes); }
-    void* cub_tmp = carve<char>(p, cub_bytes + 1);
-    Box6* leaf_box = carve<Box6>(p, L); Box6* node_box = carve<Box6>(p, L);
-    Box6* cbox_a = carve<Box6>(p, L); Box6* cbox_b = carve<Box6>(p, L);
-    unsigned long long* leaf_key = carve<unsigned long long>(p, L);
-    int2* child = carve<int2>(p, L); int2* fr_a = carve<int2>(p, L); int2* fr_b = carve<int2>(p, L);
-    int* parent_internal = carve<int>(p, L); int* parent_leaf = carve<int>(p, L); int* arrived = carve<int>(p, L);
-    int* counters = carve<int>(p, 64);
+// Scratch of one build over n primitives grouped into L leaves: the sort of the front, then the leaves and the clusters / binary nodes of
+// the back.  The back reuses the front's unsorted keys and ids.
+struct BuildScratch {
+    unsigned *keys, *keys2; int *ids, *ids2;
+    void* cub_tmp; size_t cub_bytes;
+    Box6 *leaf_box, *node_box, *cbox_a, *cbox_b;
+    unsigned long long* leaf_key;
+    int2 *child, *fr_a, *fr_b;
+    int *parent_internal, *parent_leaf, *arrived, *counters;
+};
 
-    double ext = 0.0;
-    float3 mlo, minv;
-    {
-        const float lo[3] = {bb_min[0], bb_min[1], bb_min[2]}, hi[3] = {bb_max[0], bb_max[1], bb_max[2]};
-        for (int k = 0; k < 3; ++k) ext = std::max(ext, (double)std::max(std::fabs(lo[k]), std::fabs(hi[k])));
-        mlo = make_float3(lo[0], lo[1], lo[2]);
-        auto inv = [](float a, float b) { return b > a ? 1023.999f / (b - a) : 0.0f; };
-        minv = make_float3(inv(lo[0], hi[0]), inv(lo[1], hi[1]), inv(lo[2], hi[2]));
-    }
-    const float slack = (float)(ext * 4e-6 + 1e-6);
+BuildScratch carveBuild(char*& p, int n, int L, int end_bit)
+{
+    BuildScratch s;
+    s.keys = carve<unsigned>(p, n); s.keys2 = carve<unsigned>(p, n);
+    s.ids = carve<int>(p, n); s.ids2 = carve<int>(p, n);
+    s.cub_bytes = cubBytes(n, end_bit);
+    s.cub_tmp = carve<char>(p, s.cub_bytes + 1);
+    s.leaf_box = carve<Box6>(p, L); s.node_box = carve<Box6>(p, L);
+    s.cbox_a = carve<Box6>(p, L); s.cbox_b = carve<Box6>(p, L);
+    s.leaf_key = carve<unsigned long long>(p, L);
+    s.child = carve<int2>(p, L); s.fr_a = carve<int2>(p, L); s.fr_b = carve<int2>(p, L);
+    s.parent_internal = carve<int>(p, L); s.parent_leaf = carve<int>(p, L); s.arrived = carve<int>(p, L);
+    s.counters = carve<int>(p, 64);
+    return s;
+}
+
+// The back of both builds, from L leaf boxes and keys in Morton order (s.leaf_box, s.leaf_key): PLOC (or the radix tree) to kPlocTop
+// clusters, the binned SAH on the host above them, and the breadth-first collapse into out_nodes[0 .. *nnodes) with links relative to
+// node_base.  Triangle leaves (leaf_model null) are the clusters of n triangles at leaf_base; a TLAS's leaf c is instance leaf_model[c].
+int buildTreeDevice(const BuildScratch& s, int L, int n, int leaf_base, const int* leaf_model, int node_base, BvhNode* out_nodes, cudaStream_t stream,
+                    int* nnodes, int* depth, std::string* why)
+{
     const int B = 256;
-    k_lbvh_keys<<<(n + B - 1) / B, B, 0, stream>>>(d_tris, t0, n, mlo, minv, keys, ids);
-    cudaError_t e = cub::DeviceRadixSort::SortPairs(cub_tmp, cub_bytes, (const unsigned*)keys, keys2, (const int*)ids, ids2, n, 0, 30, stream);
-    if (e != cudaSuccess) return e;
-    k_lbvh_leaves<<<(L + B - 1) / B, B, 0, stream>>>(d_tris, keys2, ids2, n, L, slack, leaf_base, btris, btid, leaf_box, leaf_key);
+    cudaError_t e = cudaSuccess;
+    size_t cub_bytes = s.cub_bytes;
     if (L == 1) {
-        k_lbvh_single<<<1, 1, 0, stream>>>(leaf_box, n, leaf_base, out_nodes);
+        if (leaf_model) k_lbvh_single<true><<<1, 1, 0, stream>>>(s.leaf_box, n, leaf_base, out_nodes, leaf_model);
+        else k_lbvh_single<<<1, 1, 0, stream>>>(s.leaf_box, n, leaf_base, out_nodes);
         *nnodes = 1; *depth = 1;
         return cudaGetLastError();
     }
     int root_node = 0;
     const char* which = getenv("PTAP_DEVICE_BUILDER");
     if (which && std::string(which) == "lbvh") {
-        k_lbvh_topology<<<(L - 1 + B - 1) / B, B, 0, stream>>>(leaf_key, L, child, parent_internal, parent_leaf);
-        e = cudaMemsetAsync(arrived, 0, (size_t)L * sizeof(int), stream);
+        k_lbvh_topology<<<(L - 1 + B - 1) / B, B, 0, stream>>>(s.leaf_key, L, s.child, s.parent_internal, s.parent_leaf);
+        e = cudaMemsetAsync(s.arrived, 0, (size_t)L * sizeof(int), stream);
         if (e != cudaSuccess) return e;
-        k_lbvh_refit<<<(L + B - 1) / B, B, 0, stream>>>(child, parent_internal, parent_leaf, leaf_box, L, node_box, arrived);
+        k_lbvh_refit<<<(L + B - 1) / B, B, 0, stream>>>(s.child, s.parent_internal, s.parent_leaf, s.leaf_box, L, s.node_box, s.arrived);
     } else {
         // PLOC: clusters (box, node) in Morton order, double-buffered across the compaction; scratch arrays of the radix-tree path are reused
-        Box6 *cb = cbox_a, *cb2 = cbox_b;
-        int *cn = parent_internal, *cn2 = parent_leaf, *nearest = arrived, *keep = reinterpret_cast<int*>(keys), *pos = ids;
+        Box6 *cb = s.cbox_a, *cb2 = s.cbox_b;
+        int *cn = s.parent_internal, *cn2 = s.parent_leaf, *nearest = s.arrived, *keep = reinterpret_cast<int*>(s.keys), *pos = s.ids;
+        int2* child = s.child;
+        Box6* node_box = s.node_box;
+        int* counters = s.counters;
         e = cudaMemsetAsync(counters + 8, 0, sizeof(int), stream);
         if (e != cudaSuccess) return e;
-        k_ploc_init<<<(L + B - 1) / B, B, 0, stream>>>(leaf_box, L, cb, cn);
+        k_ploc_init<<<(L + B - 1) / B, B, 0, stream>>>(s.leaf_box, L, cb, cn);
         int m = L, rounds = 0;
         const char* top_env = getenv("PTAP_PLOC_TOP");
         const int top = top_env ? atoi(top_env) : kPlocTop;       // clusters handed to the host's SAH build of the upper levels (0: PLOC to the root)
@@ -478,7 +491,7 @@ int buildMeshBvhDevice(const TriRec* d_tris, int t0, int t1, const float* bb_min
             const int g = (m + B - 1) / B;
             k_ploc_nearest<<<g, B, 0, stream>>>(cb, m, nearest);
             k_ploc_merge<<<g, B, 0, stream>>>(cb, cn, nearest, m, child, node_box, counters + 8, keep);
-            e = cub::DeviceScan::ExclusiveSum(cub_tmp, cub_bytes, keep, pos, m, stream);
+            e = cub::DeviceScan::ExclusiveSum(s.cub_tmp, cub_bytes, keep, pos, m, stream);
             if (e != cudaSuccess) return e;
             k_ploc_compact<<<g, B, 0, stream>>>(cb, cn, keep, pos, m, cb2, cn2);
             int last[2];
@@ -524,28 +537,234 @@ int buildMeshBvhDevice(const TriRec* d_tris, int t0, int t1, const float* bb_min
     // breadth-first collapse from the binary root: it becomes 4-wide node 0
     const int2 root = make_int2(root_node, 0);
     const int init[2] = {1, 0};
-    e = cudaMemcpyAsync(fr_a, &root, sizeof root, cudaMemcpyHostToDevice, stream);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(counters, init, sizeof init, cudaMemcpyHostToDevice, stream);
+    e = cudaMemcpyAsync(s.fr_a, &root, sizeof root, cudaMemcpyHostToDevice, stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(s.counters, init, sizeof init, cudaMemcpyHostToDevice, stream);
     if (e != cudaSuccess) return e;
     int nfrontier = 1, levels = 0;
-    int2 *cur = fr_a, *nxt = fr_b;
+    int2 *cur = s.fr_a, *nxt = s.fr_b;
     while (nfrontier > 0) {
         ++levels;
-        k_lbvh_collapse<<<(nfrontier + B - 1) / B, B, 0, stream>>>(child, node_box, leaf_box, n, leaf_base, cur, nfrontier, nxt, counters, node_base, out_nodes);
+        const int g = (nfrontier + B - 1) / B;
+        if (leaf_model) k_lbvh_collapse<true><<<g, B, 0, stream>>>(s.child, s.node_box, s.leaf_box, n, leaf_base, cur, nfrontier, nxt, s.counters, node_base, out_nodes, leaf_model);
+        else k_lbvh_collapse<<<g, B, 0, stream>>>(s.child, s.node_box, s.leaf_box, n, leaf_base, cur, nfrontier, nxt, s.counters, node_base, out_nodes);
         int host_counters[2];
-        e = cudaMemcpyAsync(host_counters, counters, sizeof host_counters, cudaMemcpyDeviceToHost, stream);
+        e = cudaMemcpyAsync(host_counters, s.counters, sizeof host_counters, cudaMemcpyDeviceToHost, stream);
         if (e == cudaSuccess) e = cudaStreamSynchronize(stream);
         if (e != cudaSuccess) return e;
         nfrontier = host_counters[1];
         *nnodes = host_counters[0];
         const int zero = 0;
-        e = cudaMemcpyAsync(counters + 1, &zero, sizeof zero, cudaMemcpyHostToDevice, stream);
+        e = cudaMemcpyAsync(s.counters + 1, &zero, sizeof zero, cudaMemcpyHostToDevice, stream);
         if (e != cudaSuccess) return e;
         std::swap(cur, nxt);
         if (levels > 200) { if (why) *why = "the 4-wide collapse exceeded 200 levels"; return cudaErrorUnknown; }
     }
     *depth = levels;
     return cudaGetLastError();
+}
+
+// ---- TLAS front: the instances of ptap_update_models -----------------------------------------------------------------------------
+
+// What k_update_instances reduces over the instances that have triangles (atomics on order-preserving bit patterns: the maxima of
+// non-negative doubles, the minimum index, the centre bounds as ordered floats).  The same values in any order of the atomics.
+struct InstanceReduce {
+    unsigned long long max_scale, max_pad, max_trans;   // bits of non-negative doubles
+    int first_bad;                                      // first model whose matrices are not inverses (INT_MAX: none)
+    unsigned clo[3], chi[3];                            // bounds of the world-box centres (orderedBits)
+};
+
+__device__ __forceinline__ unsigned orderedBits(float f)
+{
+    const unsigned u = __float_as_uint(f);
+    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
+__device__ __forceinline__ float fromOrderedBits(unsigned u) { return __uint_as_float((u & 0x80000000u) ? (u & 0x7fffffffu) : ~u); }
+
+template <typename T> __device__ __forceinline__ T warpMax(T v) { for (int o = 16; o; o >>= 1) { const T w = __shfl_xor_sync(~0u, v, o); v = w > v ? w : v; } return v; }
+template <typename T> __device__ __forceinline__ T warpMin(T v) { for (int o = 16; o; o >>= 1) { const T w = __shfl_xor_sync(~0u, v, o); v = w < v ? w : v; } return v; }
+
+// bits of a non-negative double for an atomic maximum; NaN (which std::max skips on the host) becomes 0
+__device__ __forceinline__ unsigned long long maxBits(double v) { return v == v ? (unsigned long long)__double_as_longlong(v) : 0ull; }
+
+// One thread per model.  Models [first, first + count) take their staged record: InstanceTrace.w2m / m2w (grid fields kept) and
+// InstanceShade; the others keep theirs.  With a BVH (nodes), every model that has triangles then gets its world box and its terms of
+// the scene constants from instanceBox (instance_math.h), the function finishBvh evaluates on the host; box / trans of a model without
+// triangles are an empty box and -1.
+__global__ void k_update_instances(InstanceTrace* __restrict__ inst, InstanceShade* __restrict__ shade, int nm, const PtapModel* __restrict__ staged,
+                                   int first, int count, const BvhNode* __restrict__ nodes, Box6* __restrict__ box, double* __restrict__ trans,
+                                   InstanceReduce* __restrict__ red)
+{
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    double scale = 0.0, pad = 0.0;
+    int bad = INT_MAX;
+    unsigned clo[3] = {~0u, ~0u, ~0u}, chi[3] = {0u, 0u, 0u};
+    if (i < nm) {
+        float W[16], M[16];
+        InstanceTrace& it = inst[i];
+        if (i >= first && i < first + count) {
+            const PtapModel& m = staged[i - first];
+            for (int k = 0; k < 16; ++k) { W[k] = m.world_to_model[k]; M[k] = m.model_to_world[k]; }
+            for (int r = 0; r < 3; ++r) { it.w2m[r] = make_float4(W[r], W[4 + r], W[8 + r], W[12 + r]); it.m2w[r] = make_float4(M[r], M[4 + r], M[8 + r], M[12 + r]); }
+            float nmx[9];
+            hm::normal_matrix(M, nmx);
+            InstanceShade sh;
+            sh.nm0 = make_float4(nmx[0], nmx[1], nmx[2], m.mat.color[0]);
+            sh.nm1 = make_float4(nmx[3], nmx[4], nmx[5], m.mat.color[1]);
+            sh.nm2 = make_float4(nmx[6], nmx[7], nmx[8], m.mat.color[2]);
+            sh.mat = make_int4(m.mat.type, 0, 0, 0);
+            shade[i] = sh;
+        } else {
+            for (int r = 0; r < 3; ++r) {
+                const float4 w = it.w2m[r], v = it.m2w[r];
+                W[r] = w.x; W[4 + r] = w.y; W[8 + r] = w.z; W[12 + r] = w.w;
+                M[r] = v.x; M[4 + r] = v.y; M[8 + r] = v.z; M[12 + r] = v.w;
+            }
+            W[3] = W[7] = W[11] = M[3] = M[7] = M[11] = 0.0f; W[15] = M[15] = 1.0f;
+        }
+        if (nodes) {
+            const int root = __float_as_int(it.grid.z);
+            Box6 b;
+            for (int k = 0; k < 3; ++k) { b.lo[k] = 3e38f; b.hi[k] = -3e38f; }
+            double t = -1.0;
+            InstanceBox ib;
+            if (root >= 0 && instanceBox(W, M, nodes[root], ib)) {
+                for (int k = 0; k < 3; ++k) {
+                    b.lo[k] = ib.lo[k]; b.hi[k] = ib.hi[k];
+                    clo[k] = chi[k] = orderedBits(0.5f * (ib.lo[k] + ib.hi[k]));
+                }
+                t = ib.trans; scale = ib.scale; pad = ib.pad;
+                if (!ib.consistent) bad = i;
+            }
+            box[i] = b; trans[i] = t;
+        }
+    }
+    if (!nodes) return;
+    const unsigned long long s = warpMax(maxBits(scale)), p = warpMax(maxBits(pad));
+    bad = warpMin(bad);
+    for (int k = 0; k < 3; ++k) { clo[k] = warpMin(clo[k]); chi[k] = warpMax(chi[k]); }
+    if ((threadIdx.x & 31) == 0) {
+        atomicMax(&red->max_scale, s); atomicMax(&red->max_pad, p); atomicMin(&red->first_bad, bad);
+        for (int k = 0; k < 3; ++k) { atomicMin(&red->clo[k], clo[k]); atomicMax(&red->chi[k], chi[k]); }
+    }
+}
+
+// Morton key of every instance's box centre inside the centre bounds (0xffffffff for instances without triangles: sorted last), and
+// max_trans over the models up to the first inconsistent one
+__global__ void k_instance_keys(const Box6* __restrict__ box, const double* __restrict__ trans, int nm, InstanceReduce* __restrict__ red,
+                                unsigned* __restrict__ keys, int* __restrict__ ids)
+{
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    unsigned long long t = 0ull;
+    if (i < nm) {
+        unsigned key = 0xffffffffu;
+        if (trans[i] >= 1.0) {
+            const Box6 b = box[i];
+            unsigned q[3];
+            for (int k = 0; k < 3; ++k) {
+                const float lo = fromOrderedBits(red->clo[k]), hi = fromOrderedBits(red->chi[k]);
+                const float inv = hi > lo ? 1023.999f / (hi - lo) : 0.0f;
+                q[k] = (unsigned)fminf(fmaxf((0.5f * (b.lo[k] + b.hi[k]) - lo) * inv, 0.0f), 1023.0f);
+            }
+            key = (expandBits(q[0]) << 2) | (expandBits(q[1]) << 1) | expandBits(q[2]);
+            if (i <= red->first_bad) t = maxBits(trans[i]);
+        }
+        keys[i] = key; ids[i] = i;
+    }
+    t = warpMax(t);
+    if ((threadIdx.x & 31) == 0) atomicMax(&red->max_trans, t);
+}
+
+__global__ void k_instance_leaves(const Box6* __restrict__ box, const unsigned* __restrict__ keys, const int* __restrict__ ids, int L,
+                                  Box6* __restrict__ leaf_box, unsigned long long* __restrict__ leaf_key)
+{
+    const int c = blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= L) return;
+    leaf_box[c] = box[ids[c]];
+    leaf_key[c] = ((unsigned long long)keys[c] << 32) | (unsigned)c;
+}
+
+}  // namespace
+
+size_t deviceBvhScratchBytes(int ntris) { return scratchBytes(ntris, (std::max(ntris, 1) + kCluster - 1) / kCluster, 30); }
+
+size_t instanceUpdateScratchBytes(int nmodels)
+{
+    const size_t n = (size_t)std::max(nmodels, 1);
+    return scratchBytes(nmodels, nmodels, 32) +                       // one leaf per instance, whatever kCluster is
+           ((n * sizeof(Box6) + 255) & ~size_t(255)) + ((n * sizeof(double) + 255) & ~size_t(255)) + 256;
+}
+
+// Builds the BLAS of one mesh (triangles [t0, t1) of the global table) into out_nodes[0 .. *nnodes) with links relative to node_base,
+// leaf-order triangles into btris / btid at [leaf_base, leaf_base + n).  Returns a cudaError_t; *depth = levels of 4-wide nodes.  When the
+// build itself gives up (not a CUDA call), *why says why.
+int buildMeshBvhDevice(const TriRec* d_tris, int t0, int t1, const float* bb_min, const float* bb_max, int node_base, BvhNode* out_nodes, int leaf_base,
+                       LeafTri* btris, int* btid, char* scratch, size_t scratch_bytes, cudaStream_t stream, int* nnodes, int* depth, std::string* why)
+{
+    const int n = t1 - t0, L = (n + kCluster - 1) / kCluster;
+    *nnodes = 0; *depth = 0;
+    if (n <= 0) return cudaSuccess;
+    if (deviceBvhScratchBytes(n) > scratch_bytes) return cudaErrorMemoryAllocation;
+    char* p = scratch;
+    const BuildScratch s = carveBuild(p, n, L, 30);
+
+    double ext = 0.0;
+    float3 mlo, minv;
+    {
+        const float lo[3] = {bb_min[0], bb_min[1], bb_min[2]}, hi[3] = {bb_max[0], bb_max[1], bb_max[2]};
+        for (int k = 0; k < 3; ++k) ext = std::max(ext, (double)std::max(std::fabs(lo[k]), std::fabs(hi[k])));
+        mlo = make_float3(lo[0], lo[1], lo[2]);
+        auto inv = [](float a, float b) { return b > a ? 1023.999f / (b - a) : 0.0f; };
+        minv = make_float3(inv(lo[0], hi[0]), inv(lo[1], hi[1]), inv(lo[2], hi[2]));
+    }
+    const float slack = (float)(ext * 4e-6 + 1e-6);
+    const int B = 256;
+    k_lbvh_keys<<<(n + B - 1) / B, B, 0, stream>>>(d_tris, t0, n, mlo, minv, s.keys, s.ids);
+    size_t cub_bytes = s.cub_bytes;
+    const cudaError_t e = cub::DeviceRadixSort::SortPairs(s.cub_tmp, cub_bytes, (const unsigned*)s.keys, s.keys2, (const int*)s.ids, s.ids2, n, 0, 30, stream);
+    if (e != cudaSuccess) return e;
+    k_lbvh_leaves<<<(L + B - 1) / B, B, 0, stream>>>(d_tris, s.keys2, s.ids2, n, L, slack, leaf_base, btris, btid, s.leaf_box, s.leaf_key);
+    return buildTreeDevice(s, L, n, leaf_base, nullptr, node_base, out_nodes, stream, nnodes, depth, why);
+}
+
+int updateInstancesDevice(InstanceTrace* inst, InstanceShade* shade, int nmodels, const PtapModel* staged, int first, int count, BvhNode* nodes,
+                          int node_base, int ninst, char* scratch, size_t scratch_bytes, cudaStream_t stream, TlasBuild* out, std::string* why)
+{
+    const int B = 256, g = (nmodels + B - 1) / B;
+    *out = TlasBuild{};
+    if (!nodes) {
+        k_update_instances<<<g, B, 0, stream>>>(inst, shade, nmodels, staged, first, count, nullptr, nullptr, nullptr, nullptr);
+        return cudaGetLastError();
+    }
+    if (instanceUpdateScratchBytes(nmodels) > scratch_bytes) return cudaErrorMemoryAllocation;
+    char* p = scratch;
+    const BuildScratch s = carveBuild(p, nmodels, nmodels, 32);
+    Box6* box = carve<Box6>(p, nmodels);
+    double* trans = carve<double>(p, nmodels);
+    InstanceReduce* red = carve<InstanceReduce>(p, 1);
+    InstanceReduce init;
+    init.max_scale = init.max_pad = 0ull;
+    { const double one = 1.0; memcpy(&init.max_trans, &one, sizeof one); }
+    init.first_bad = INT_MAX;
+    for (int k = 0; k < 3; ++k) { init.clo[k] = ~0u; init.chi[k] = 0u; }
+    cudaError_t e = cudaMemcpyAsync(red, &init, sizeof init, cudaMemcpyHostToDevice, stream);
+    if (e != cudaSuccess) return e;
+    k_update_instances<<<g, B, 0, stream>>>(inst, shade, nmodels, staged, first, count, nodes, box, trans, red);
+    k_instance_keys<<<g, B, 0, stream>>>(box, trans, nmodels, red, s.keys, s.ids);
+    size_t cub_bytes = s.cub_bytes;
+    e = cub::DeviceRadixSort::SortPairs(s.cub_tmp, cub_bytes, (const unsigned*)s.keys, s.keys2, (const int*)s.ids, s.ids2, nmodels, 0, 32, stream);
+    if (e != cudaSuccess) return e;
+    InstanceReduce r;
+    e = cudaMemcpyAsync(&r, red, sizeof r, cudaMemcpyDeviceToHost, stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(stream);
+    if (e != cudaSuccess) return e;
+    memcpy(&out->max_scale, &r.max_scale, sizeof(double)); memcpy(&out->max_pad, &r.max_pad, sizeof(double)); memcpy(&out->max_trans, &r.max_trans, sizeof(double));
+    out->consistent = r.first_bad == INT_MAX;
+    out->root = -1;
+    if (ninst == 0) return cudaSuccess;
+    k_instance_leaves<<<(ninst + B - 1) / B, B, 0, stream>>>(box, s.keys2, s.ids2, ninst, s.leaf_box, s.leaf_key);
+    e = (cudaError_t)buildTreeDevice(s, ninst, ninst, 0, s.ids2, node_base, nodes + node_base, stream, &out->nnodes, &out->depth, why);
+    if (e == cudaSuccess) out->root = node_base;
+    return e;
 }
 
 }  // namespace ptap

@@ -4,6 +4,8 @@
 #pragma once
 #include <cmath>
 
+#include <cuda_runtime.h>
+
 namespace ptap { namespace hm {
 
 struct V3 { float x, y, z; };
@@ -24,8 +26,8 @@ inline V3 mat4_mul(const float* m, V3 v, float w)
 }
 
 // rows of transpose(inverse(mat3(M))) as utility.h:82-88 evaluates it (inverse: detail/type_mat3x3.inl:37-56).
-// out[3*r + k] multiplies n[k] in component r.
-inline void normal_matrix(const float* M, float out[9])
+// out[3*r + k] multiplies n[k] in component r.  Also compiled for the device (k_update_instances, -fmad=false): the same bits.
+__host__ __device__ inline void normal_matrix(const float* M, float out[9])
 {
     auto m = [&](int c, int r) { return M[4 * c + r]; };
     const float ood = 1.0f / (+m(0, 0) * (m(1, 1) * m(2, 2) - m(2, 1) * m(1, 2))

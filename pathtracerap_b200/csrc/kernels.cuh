@@ -71,6 +71,17 @@ size_t deviceBvhScratchBytes(int ntris);
 int buildMeshBvhDevice(const TriRec* d_tris, int t0, int t1, const float* bb_min, const float* bb_max, int node_base, BvhNode* out_nodes, int leaf_base,
                        LeafTri* btris, int* btid, char* scratch, size_t scratch_bytes, cudaStream_t stream, int* nnodes, int* depth,
                        std::string* why);
+// ptap_update_models: models [first, first + count) take the staged records (device copies) in their InstanceTrace (grid fields kept) and
+// InstanceShade.  With a BVH (nodes non-null), the TLAS over the instances' world boxes is then built at nodes + node_base (ninst = models
+// with triangles) and the scene-constant terms are reduced (TlasBuild), all from the same per-instance function as finishBvh.
+struct TlasBuild {
+    int root = -1, nnodes = 0, depth = 0;       // root node index (-1: no instance has triangles), 4-wide nodes and levels of the TLAS
+    double max_scale = 0.0, max_pad = 0.0, max_trans = 1.0;
+    bool consistent = true;
+};
+size_t instanceUpdateScratchBytes(int nmodels);
+int updateInstancesDevice(InstanceTrace* inst, InstanceShade* shade, int nmodels, const PtapModel* staged, int first, int count, BvhNode* nodes,
+                          int node_base, int ninst, char* scratch, size_t scratch_bytes, cudaStream_t stream, TlasBuild* out, std::string* why);
 
 // grid_device.cu: Scene::addMeshesToGrid on the device, one mesh's grid at a time
 int gridDeviceCount(const float* d_pos, int t0, int n, const float bb_min[3], const float width[3], const int gd[3], int* d_count, int* d_offset,

@@ -112,6 +112,17 @@ class Renderer:
         self._check(N.lib().ptap_upload_scene(self.h, C.byref(v)), "upload_scene")
         self._check(N.lib().ptap_build_accel(self.h, self.accel), "build_accel")
 
+    def update_models(self, models, first: int = 0):
+        """Replace models [first, first + len(models)) of the uploaded scene (transforms and material; ptap_update_models): the
+        instance records and the TLAS are rebuilt on the GPU, the meshes' BVHs stay.  `models` is an N.MODEL array, or a Scene for all
+        of its models.  Afterwards the renderer traces and renders exactly as one that uploaded the scene with these models."""
+        if isinstance(models, Scene):
+            models = models.models
+        if not isinstance(models, np.ndarray) or models.dtype != N.MODEL:
+            raise N.PtapError(f"update_models: models must be an array of dtype MODEL, got {getattr(models, 'dtype', type(models).__name__)}")
+        models = np.ascontiguousarray(models.reshape(-1))
+        self._check(N.lib().ptap_update_models(self.h, N.ptr(models), int(first), len(models)), "update_models")
+
     def frame_begin(self):
         """Start of a renderLoop: zero film, forget the first-hit cache, zero the counters."""
         self._check(N.lib().ptap_frame_begin(self.h), "frame_begin")

@@ -153,7 +153,8 @@ class Scene:
         raise AttributeError(name)
 
     def set_models(self, models):
-        """Overwrite the models in place (material / transform edits before allocateOnGPU, SURVEY.md A.3b)."""
+        """Overwrite the models in place (material / transform edits, SURVEY.md A.3b).  A renderer that has uploaded the scene takes
+        the edits through Renderer.update_models."""
         models = np.ascontiguousarray(models, N.MODEL)
         v = self.view()
         if len(models) != v.nmodels:

@@ -3,8 +3,10 @@
     python tools/sass_diff.py OLD/libptap.so NEW/libptap.so
 
 Instructions are compared without their encodings' address comments and blank lines.  Names are normalised for what does not change
-code: the hash of anonymous namespaces (it depends on the build directory) and the ANY = false parameter that k_trace_bvh gained with the
-any-hit mode (`k_trace_bvh<UV, COUNT>` before, `<UV, COUNT, false>` after).  Exit status 1 when a kernel of OLD is missing or differs."""
+code: the hash of anonymous namespaces (it depends on the build directory), the ANY = false parameter that k_trace_bvh gained with the
+any-hit mode (`k_trace_bvh<UV, COUNT>` before, `<UV, COUNT, false>` after), and the INST = false parameter and trailing `leaf_model`
+argument that k_lbvh_collapse and k_lbvh_single gained with the device TLAS (compared by their demangled names without either).  Exit
+status 1 when a kernel of OLD is missing or differs."""
 import re
 import subprocess
 import sys
@@ -26,6 +28,9 @@ def kernels(lib):
 
 
 def norm(name):
+    if re.search(r"k_lbvh_(collapse|single)(ILb0EEEv|E)", name):            # the triangle-leaf instantiation, before and after
+        d = subprocess.run(["c++filt", name], capture_output=True, text=True, check=True).stdout.strip()
+        return re.sub(r", int const\*\)$", ")", re.sub(r"^void ", "", d).replace("<false>", ""))
     name = re.sub(r"_GLOBAL__N__[0-9a-f]+_", "_GLOBAL__N__", name)
     return re.sub(r"(k_trace_bvhILb[01]ELb[01]E)Lb0EE", r"\1E", name)
 
