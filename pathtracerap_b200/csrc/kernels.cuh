@@ -18,13 +18,10 @@ constexpr int kScanBlock = 256, kScanSlots = 2048, kScanTiles = kScanSlots / kSh
 constexpr int kGenBlock = 256;
 constexpr int kMaxLanes = 8, kDefaultLanes = 4, kSmallFrameLanes = 8;   // wavefronts in flight per context (api.cu: multi-lane rendering)
 constexpr int kTraceBatch = 32;      // rays a warp takes from the work-stealing cursor per atomic
-constexpr int kVoteTri = 8, kVoteInst = 6, kVoteRefill = 8;
-constexpr int kVoteGrid = 5;         // same for k_trace_grid (one threshold for all of its states)   // state-machine thresholds of k_trace_bvh (trace_bvh.cu)
+constexpr int kVoteTri = 8, kVoteInst = 6, kVoteRefill = 8;   // state-machine thresholds of k_trace_bvh (trace_bvh.cu)
+constexpr int kVoteGrid = 5;         // same for k_trace_grid (one threshold for all of its states)
+constexpr unsigned kFull = 0xffffffffu;   // every lane of a warp
 
-// World distance of the hit at model-space parameter t of model `im` along the stored ray (bo, bd), exactly as the reference computes
-// it (Renderer.cpp:381-382 ray set-up, :388-391 conversion).  k_trace_bvh only carries an approximate distance while traversing
-// (it needs the exact one just to break near-ties); the consumers of a hit record (k_shade, k_resolve_hits) evaluate this function,
-// at full SIMT efficiency, instead of the traversal doing it with a handful of active lanes.
 __device__ __forceinline__ unsigned long long globalTimerNs()
 {
     unsigned long long t;
@@ -32,6 +29,44 @@ __device__ __forceinline__ unsigned long long globalTimerNs()
     return t;
 }
 
+// A warp's share of a work-stealing cursor: the items [w_next, w_end) of the batch it took last.  Every lane of the warp calls both steps.
+struct WarpBatch {
+    int w_next = 0, w_end = 0;
+    bool exhausted = false;                      // the cursor has passed n: nothing left to fetch
+    // the warp's batch is used up: take the next `batch` items (one atomic per warp)
+    __device__ __forceinline__ void fetch(unsigned int* cursor, int batch, int n)
+    {
+        if (w_next >= w_end && !exhausted) {
+            unsigned b = 0;
+            if ((threadIdx.x & 31) == 0) b = atomicAdd(cursor, (unsigned)batch);
+            b = __shfl_sync(kFull, b, 0);
+            if (b >= (unsigned)n) { exhausted = true; w_next = w_end = n; }
+            else { w_next = (int)b; w_end = min((int)b + batch, n); }
+        }
+    }
+    // the lanes of `free` (ballot of `mine`) take the next items in lane order: true when this lane gets one (`item`); then every lane calls
+    // advance() past the items taken
+    __device__ __forceinline__ bool claim(unsigned free, bool mine, int& item) const
+    {
+        const int rank = __popc(free & ((1u << (threadIdx.x & 31)) - 1u));
+        item = w_next + rank;
+        return mine && rank < w_end - w_next;
+    }
+    __device__ __forceinline__ void advance(unsigned free) { w_next += min(__popc(free), w_end - w_next); }
+};
+
+// counting builds: the warp's sum of v added to *total by lane 0
+__device__ __forceinline__ void warpTotalAdd(unsigned long long* total, unsigned long long v)
+{
+#pragma unroll
+    for (int d = 16; d > 0; d >>= 1) v += __shfl_xor_sync(kFull, v, d);
+    if ((threadIdx.x & 31) == 0) atomicAdd(total, v);
+}
+
+// World distance of the hit at model-space parameter t of model `im` along the stored ray (bo, bd), exactly as the reference computes
+// it (Renderer.cpp:381-382 ray set-up, :388-391 conversion).  k_trace_bvh only carries an approximate distance while traversing
+// (it needs the exact one just to break near-ties); the consumers of a hit record (k_shade, k_resolve_hits) evaluate this function,
+// at full SIMT efficiency, instead of the traversal doing it with a handful of active lanes.
 __device__ __forceinline__ float exactHitDistance(const SceneDev& sc, V3 bo, V3 bd, int im, float t)
 {
     const InstanceTrace* __restrict__ inst = &sc.inst[im];

@@ -48,7 +48,6 @@ namespace {
 #endif
 constexpr int kFullBatch = PTAP_EMU_FULL_BATCH;   // list entries a warp of k_emu_full takes per fetch: few, so that a short list spreads over all warps (the kernel is latency-bound)
 constexpr int kFullHits = 20;                 // hits of a (ray, model) that k_emu_full keeps in shared memory (46 KB per CTA with the stack)
-constexpr int kEmuStack = 12;                 // traversal-stack entries per ray in shared memory (as k_trace_bvh)
 constexpr int kReplayBlock = 128, kReplayBatch = 32;   // k_emu_tail: threads per CTA, queue entries per cursor fetch
 constexpr int kSetupBlock = 128;                      // k_emu_setup
 #ifndef PTAP_EMU_SETUP_STEPS
@@ -77,7 +76,6 @@ k_trace_emu(SceneDev sc, const float4* __restrict__ O, const float4* __restrict_
     if (blockIdx.x == 0 && threadIdx.x == 0 && n_fixed < 0) st->rays_traced += (unsigned long long)n;
     if (stamp && threadIdx.x == 0) atomicMin(stamp, globalTimerNs());
     unsigned int* cursor = &st->fetch[round];
-    const int lane = threadIdx.x & 31;
     unsigned long long tot_x = 0, tot_z = 0;
     int4 cnt = make_int4(0, 0, 0, 0);      // counting build: nodes visited, (voxels replayed: launch 2), triangles tested
 
@@ -90,11 +88,9 @@ k_trace_emu(SceneDev sc, const float4* __restrict__ O, const float4* __restrict_
         return;
     }
 
-    int sp = 0;
-    __shared__ int s_stack[kEmuStack * kTraceBlock];       // [entry][thread]: a warp-wide push / pop is one wavefront (trace_bvh.cu)
-    int l_stack[kBvhStack - kEmuStack];
-    auto push = [&](int v) { if (sp < kEmuStack) s_stack[sp * kTraceBlock + threadIdx.x] = v; else l_stack[sp - kEmuStack] = v; ++sp; };
-    auto pop = [&]() { --sp; return sp < kEmuStack ? s_stack[sp * kTraceBlock + threadIdx.x] : l_stack[sp - kEmuStack]; };
+    __shared__ int s_stack[kSmemStack * kTraceBlock];
+    int l_stack[kBvhStack - kSmemStack];
+    SplitStack stack(s_stack, l_stack);
     // the hits of the instance being traversed and of the nearest instance so far: two buffers [buffer][hit][thread] that swap roles
     __shared__ int s_id[2 * kEmuHits * kTraceBlock];
     __shared__ float s_t[2 * kEmuHits * kTraceBlock];
@@ -113,48 +109,28 @@ k_trace_emu(SceneDev sc, const float4* __restrict__ O, const float4* __restrict_
     float tmin = 0.0f, tmax = 0.0f;
     float g_dist = kFloatMax, g_t = 0.0f;
     int g_model = -1, g_tri = -1;
-    int w_next = 0, w_end = 0;
-    bool exhausted = false;
+    WarpBatch work;
     const int vote_tri = sc.vote_tri, vote_inst = sc.vote_inst, vote_refill = sc.vote_refill;
 
     for (;;) {
         // ---- (1) inner nodes: as k_trace_bvh, except that inside an instance the interval never shrinks (every hit is wanted)
         if (node >= 0) {
             int key[4], lnk[4];
-            nodeChildren(reinterpret_cast<const char*>(&sc.nodes[node]), ro, rinv, near_off, tmin, tmax, key, lnk);
+            nodeChildren<true>(reinterpret_cast<const char*>(&sc.nodes[node]), ro, rinv, near_off, tmin, tmax, key, lnk);
             if (COUNT) cnt.x++;
-            if (key[3] != 0x7f800000) push(lnk[3]);
-            if (key[2] != 0x7f800000) push(lnk[2]);
-            if (key[1] != 0x7f800000) push(lnk[1]);
-            if (key[0] != 0x7f800000) node = lnk[0]; else node = pop();
+            node = stack.descend(key, lnk);
         }
         // ---- (2) who waits for what
-        const unsigned code = ~(unsigned)node;
-        const unsigned state = min(code >> 29, 4u);             // 0 tri, 1 enter, 2 exit, 3 done, 4 inner
-        const bool live = state != 3u || i >= 0 || !exhausted;
-        const unsigned sum = __reduce_add_sync(kFull, live ? 1u << (6u * state) : 0u);
-        if (sum == 0u) break;
-        const int n_tri = sum & 63u, n_enter = (sum >> 6) & 63u, n_exit = (sum >> 12) & 63u, n_done = (sum >> 18) & 63u, n_inner = (sum >> 24) & 63u;
-        const bool s_tri = state == 0u, s_enter = state == 1u, s_exit = state == 2u, s_done = state == 3u;
+        const LaneVote vt = laneVote(node, i >= 0 || !work.exhausted);
+        if (vt.n_all == 0u) break;
+        const unsigned code = vt.code;
 
         // ---- (3a) one triangle of the held leaf: the reference's predicate (Renderer.cpp:174-201), every hit recorded
-        if (s_tri && n_tri >= min(vote_tri, n_inner)) {
-            const int k = (int)(code >> 3);
-            const F8 ta = ldg8(&sc.bvh_tris[k]), tb = ldg8(reinterpret_cast<const char*>(&sc.bvh_tris[k]) + 32);
+        if (vt.tri && vt.n_tri >= min(vote_tri, vt.n_inner)) {
+            const TriTest h = leafTriangle(sc, (int)(code >> 3), ro, rd);
             if (COUNT) cnt.z++;
-            const V3 v0 = v3(ta.v[0], ta.v[1], ta.v[2]), v0v1 = v3(ta.v[3], ta.v[4], ta.v[5]), v0v2 = v3(ta.v[6], ta.v[7], tb.v[0]);
-            const V3 pvec = xcross(rd, v0v2);
-            const float det = xdot(v0v1, pvec);
-            const float invDet = xdiv(1.0f, det);
-            const V3 tvec = xsub(ro, v0);
-            const float u = xmul(xdot(tvec, pvec), invDet);
-            const V3 qvec = xcross(tvec, v0v1);
-            const float v = xmul(xdot(rd, qvec), invDet);
-            const float t = xmul(xdot(v0v2, qvec), invDet);
-            const bool reject = (xabs(xsub(det, 0.0f)) < kEpsilon) | (u < (0.0f - kEpsilon)) | (u > (1.0f + kEpsilon)) |
-                                (v < (0.0f - kEpsilon)) | (xadd(u, v) > (1.0f + kEpsilon)) | (t < (0.0f - kEpsilon));
-            if (!reject) {
-                const int id = __float_as_int(tb.v[1]);
+            if (!h.reject) {
+                const int id = h.id; const float t = h.t;
                 if (nh < kEmuHits) {
                     const int slot = ((cur * kEmuHits + nh) * kTraceBlock) + threadIdx.x;
                     s_id[slot] = id; s_t[slot] = t;
@@ -162,64 +138,41 @@ k_trace_emu(SceneDev sc, const float4* __restrict__ O, const float4* __restrict_
                 ++nh;
                 if (t < c_t || (t == c_t && c_tri >= 0 && id < c_tri)) { c_t = t; c_tri = id; }      // brute force in index order
             }
-            if (code & 7u) node = (int)~(code + 7u); else node = pop();
+            if (code & 7u) node = (int)~(code + 7u); else node = stack.pop();
         }
         // ---- (3b) TLAS leaf: enter instance `im` (Renderer.cpp:381-384)
-        if (s_enter && n_enter >= min(vote_inst, n_inner)) {
+        if (vt.enter && vt.n_enter >= min(vote_inst, vt.n_inner)) {
             const int im = (int)(code & kIndexMask);
             const InstanceTrace* __restrict__ inst = &sc.inst[im];
-            const float4 w0 = ldg4(&inst->w2m[0]), w1 = ldg4(&inst->w2m[1]), w2 = ldg4(&inst->w2m[2]);
-            ro = xmat4(w0, w1, w2, bo, 1.0f);                                   // Renderer.cpp:381
-            const V3 dm = xmat4(w0, w1, w2, bd, 0.0f);
-            const float mlen = xsqrt(xdot(dm, dm));
-            rd = xscale(dm, xdiv(1.0f, mlen));                                  // glm::normalize, Renderer.cpp:382
-            rinv = v3(safeInv(rd.x), safeInv(rd.y), safeInv(rd.z));
-            near_off = nearOffsets(rd);
-            const float wil = rsqrtf(bd.x * bd.x + bd.y * bd.y + bd.z * bd.z);
-            tmin = -(kEpsilon + 1e-4f);                                         // the predicate accepts t >= -EPSILON
+            const float mscale = enterInstance(inst, bo, bd, ro, rd, rinv, near_off);
+            tmin = kModelTmin;
             tmax = 3.0e38f;                                                     // all hits: a far one can keep the walk going until it meets a near one
             nh = 0; c_t = kFloatMax; c_tri = -1;
-            push(__float_as_int(__fdividef(1.0f, mlen * wil)));                  // world distance per unit of model-space t, for the exit step
-            push((int)~(kExitBit | (unsigned)im));
+            stack.push(__float_as_int(__fdividef(1.0f, mscale)));                  // world distance per unit of model-space t, for the exit step
+            stack.push((int)~(kExitBit | (unsigned)im));
             node = __float_as_int(__ldg(&inst->grid.z));                        // BLAS root of the instance's mesh
         }
         // ---- (3c) marker popped: leave instance `im`; nearest-model decision (Renderer.cpp:388-398) exactly as k_trace_bvh makes it
-        if (s_exit && n_exit >= min(vote_inst, n_inner)) {
+        if (vt.exit && vt.n_exit >= min(vote_inst, vt.n_inner)) {
             const int im = (int)(code & kIndexMask);
-            const float ascale = __int_as_float(pop());
-            const float cb = sc.c_pad + 1e-4f * (fabsf(bo.x) + fabsf(bo.y) + fabsf(bo.z));
+            const float ascale = __int_as_float(stack.pop());
+            const float cb = rankSlack(sc, bo);
             const bool amb = c_tri >= 0 && c_t < 0.0f && nh >= 2;
             if (amb) ++n_amb;
-            if (c_tri >= 0) {
-                const float a = fabsf(c_t * ascale);
-                const float a_lo = a - (fabsf(a) * sc.tie + cb), a_hi = a + (fabsf(a) * sc.tie + cb);
-                const float g_lo = g_dist - (g_dist * sc.tie + cb), g_hi = g_dist + (g_dist * sc.tie + cb);
-                bool take;
-                float nd = a;
-                if (a_hi < g_lo && a_hi < 0.99f * kFloatMax) take = true;
-                else if (g_model >= 0 && a_lo > g_hi) take = false;
-                else {                                                           // near-tie, or no usable bound: the reference's comparison
-                    const float dn = exactHitDistance(sc, bo, bd, im, c_t);
-                    const float dg = g_model >= 0 ? exactHitDistance(sc, bo, bd, g_model, g_t) : kFloatMax;
-                    take = dg > dn || (dg == dn && g_model >= 0 && im < g_model);   // Renderer.cpp:393 in model order
-                    nd = dn;
-                    if (!take && g_model >= 0) g_dist = dg;
-                }
-                if (take) {
-                    g_dist = nd; g_model = im; g_tri = c_tri; g_t = c_t;
-                    nh_best = nh; cur ^= 1;                                      // the buffer just filled is kept; the next instance fills the other
-                    best_amb = amb;
-                }
+            if (c_tri >= 0 && takeInstance<false>(sc, bo, bd, cb, im, c_t, ascale, g_model, g_t, g_dist)) {
+                g_model = im; g_tri = c_tri; g_t = c_t;
+                nh_best = nh; cur ^= 1;                                          // the buffer just filled is kept; the next instance fills the other
+                best_amb = amb;
             }
             nh = 0; c_t = kFloatMax; c_tri = -1;
             ro = bo; rinv = winv; near_off = wnear_off;
             tmin = sc.tmin_world; tmax = worldBound(g_dist, sc.prune, cb);
-            node = pop();
+            node = stack.pop();
         }
         // ---- (3d) retire finished rays, refill the lanes from the warp's batch
-        if (n_done > 0 && n_done >= min(vote_refill, n_inner)) {
-            const unsigned m_done = __ballot_sync(kFull, s_done && live);
-            if (s_done && i >= 0) {
+        if (vt.n_done > 0 && vt.n_done >= min(vote_refill, vt.n_inner)) {
+            const unsigned m_done = __ballot_sync(kFull, vt.done && vt.live);
+            if (vt.done && i >= 0) {
                 const bool found = g_model >= 0;
                 hit[i] = make_float4(found ? -1.0f : kFloatMax, __int_as_float(found ? g_tri : -1), __int_as_float(found ? g_model : -1), g_t);
                 emu.n[i] = !found ? 0 : n_amb > (best_amb ? 1 : 0) ? kEmuHits + 1 : nh_best;      // > kEmuHits: not replayed, the walk answers
@@ -233,17 +186,10 @@ k_trace_emu(SceneDev sc, const float4* __restrict__ O, const float4* __restrict_
                 if (COUNT) { if (counts) counts[i] = cnt; tot_x += cnt.x; tot_z += cnt.z; }
                 i = -1;
             }
-            if (w_next >= w_end && !exhausted) {
-                unsigned b = 0;
-                if (lane == 0) b = atomicAdd(cursor, (unsigned)sc.batch);
-                b = __shfl_sync(kFull, b, 0);
-                if (b >= (unsigned)n) { exhausted = true; w_next = w_end = n; }
-                else { w_next = (int)b; w_end = min((int)b + sc.batch, n); }
-            }
-            const int avail = w_end - w_next;
-            const int rank = __popc(m_done & ((1u << lane) - 1u));
-            if (s_done && live && rank < avail) {
-                i = w_next + rank;
+            work.fetch(cursor, sc.batch, n);
+            int next;
+            if (work.claim(m_done, vt.done && vt.live, next)) {
+                i = next;
                 const float4 o4 = O[i], d4 = D[i];
                 bo = v3(o4); bd = v3(d4);
                 const float il = rsqrtf(bd.x * bd.x + bd.y * bd.y + bd.z * bd.z);
@@ -254,18 +200,14 @@ k_trace_emu(SceneDev sc, const float4* __restrict__ O, const float4* __restrict_
                 g_dist = kFloatMax; g_model = -1; g_tri = -1; g_t = 0.0f;
                 nh = 0; nh_best = 0; c_t = kFloatMax; c_tri = -1; n_amb = 0; best_amb = false;
                 if (COUNT) cnt = make_int4(0, 0, 0, 0);
-                sp = 0; push(kDone);
+                stack.sp = 0; stack.push(kDone);
                 node = sc.tlas_root;
             }
-            w_next += min(__popc(m_done), avail);
+            work.advance(m_done);
         }
     }
     if (stamp && (threadIdx.x & 31) == 0) atomicMax(stamp + 1, globalTimerNs());
-    if (COUNT) {
-#pragma unroll
-        for (int d = 16; d > 0; d >>= 1) { tot_x += __shfl_xor_sync(kFull, tot_x, d); tot_z += __shfl_xor_sync(kFull, tot_z, d); }
-        if (lane == 0) { atomicAdd(&st->count_nodes, tot_x); atomicAdd(&st->count_tris, tot_z); }
-    }
+    if (COUNT) { warpTotalAdd(&st->count_nodes, tot_x); warpTotalAdd(&st->count_tris, tot_z); }
 }
 
 // ---- launches 2 and 3: replay the walk of the nearest model over its hits (Renderer.cpp:238-360) -----------------------------------------
@@ -286,6 +228,35 @@ struct Replay {
     float tmx, tmy, tmz, dx, dy, dz, w_t, t_star;
     bool inter, passed;
 };
+
+// the walk leaves the model: more than two voxels past the last voxel that listed a hit triangle (Renderer.cpp:326-329)
+__device__ __forceinline__ bool pastLastHit(const Replay& r)
+{
+    return r.inter && (abs(r.cx - r.ix) > 2 || abs(r.cy - r.iy) > 2 || abs(r.cz - r.iz) > 2);
+}
+
+// one DDA step to the next voxel (Renderer.cpp:331-357, without branches); true when the walk leaves the grid
+__device__ __forceinline__ bool ddaStep(Replay& r, int GX, int GY, int GZ)
+{
+    const bool px = r.gpos & (1u << 9), py = r.gpos & (1u << 19), pz = r.gpos & (1u << 29);
+    const bool sx = r.tmx < r.tmy && r.tmx < r.tmz, sy = !sx && r.tmy < r.tmz;
+    r.ix += sx ? (px ? 1 : -1) : 0; r.iy += sy ? (py ? 1 : -1) : 0; r.iz += (sx || sy) ? 0 : (pz ? 1 : -1);
+    const float tsel = sx ? r.tmx : sy ? r.tmy : r.tmz;
+    const int isel = sx ? r.ix : sy ? r.iy : r.iz, lim = sx ? (px ? GX : -1) : sy ? (py ? GY : -1) : (pz ? GZ : -1);
+    if (isel == lim || tsel >= kFloatMax) return true;
+    r.tmx = sx ? xadd(r.tmx, r.dx) : r.tmx; r.tmy = sy ? xadd(r.tmy, r.dy) : r.tmy; r.tmz = (sx || sy) ? r.tmz : xadd(r.tmz, r.dz);
+    return false;
+}
+
+// the box (ulo, uhi) around the voxel boxes of a replay's hits: start empty, then add each hit's box [lj, hj]
+constexpr unsigned kEmptyLo = 0x1ffu | (0x1ffu << 10) | (0x1ffu << 20), kEmptyHi = 0u;
+__device__ __forceinline__ void unionBox(unsigned& ulo, unsigned& uhi, unsigned lj, unsigned hj)
+{
+    if ((((hj | kGuard) - lj) & kGuard) == kGuard) {                    // listed somewhere (lo <= hi on every axis)
+        ulo = min(ulo & 0x1ffu, lj & 0x1ffu) | min(ulo & (0x1ffu << 10), lj & (0x1ffu << 10)) | min(ulo & (0x1ffu << 20), lj & (0x1ffu << 20));
+        uhi = max(uhi & 0x1ffu, hj & 0x1ffu) | max(uhi & (0x1ffu << 10), hj & (0x1ffu << 10)) | max(uhi & (0x1ffu << 20), hj & (0x1ffu << 20));
+    }
+}
 
 // one voxel of the walk; true when the replay is over (r.w_tri / r.w_t hold the walk's answer so far)
 template <int BURST = kBurst>
@@ -316,17 +287,9 @@ __device__ __forceinline__ bool replayStep(Replay& r, int GX, int GY, int GZ, co
     if (r.w_t == r.t_star) finished = true;
     else {
         if (any) { r.cx = r.ix; r.cy = r.iy; r.cz = r.iz; r.inter = true; }
-        if (r.inter && (abs(r.cx - r.ix) > 2 || abs(r.cy - r.iy) > 2 || abs(r.cz - r.iz) > 2)) finished = true;       // Renderer.cpp:326-329
+        if (pastLastHit(r)) finished = true;
         else if (r.passed) finished = true;         // no voxel ahead lists a hit triangle: the walk ends with what it has
-        else {                                                                                                       // Renderer.cpp:331-357, without branches
-            const bool px = r.gpos & (1u << 9), py = r.gpos & (1u << 19), pz = r.gpos & (1u << 29);
-            const bool sx = r.tmx < r.tmy && r.tmx < r.tmz, sy = !sx && r.tmy < r.tmz;
-            r.ix += sx ? (px ? 1 : -1) : 0; r.iy += sy ? (py ? 1 : -1) : 0; r.iz += (sx || sy) ? 0 : (pz ? 1 : -1);
-            const float tsel = sx ? r.tmx : sy ? r.tmy : r.tmz;
-            const int isel = sx ? r.ix : sy ? r.iy : r.iz, lim = sx ? (px ? GX : -1) : sy ? (py ? GY : -1) : (pz ? GZ : -1);
-            if (isel == lim || tsel >= kFloatMax) finished = true;
-            else { r.tmx = sx ? xadd(r.tmx, r.dx) : r.tmx; r.tmy = sy ? xadd(r.tmy, r.dy) : r.tmy; r.tmz = (sx || sy) ? r.tmz : xadd(r.tmz, r.dz); }
-        }
+        else finished = ddaStep(r, GX, GY, GZ);
     }
     ++r.k;
     // Voxels outside the box around the hits list no hit triangle: nothing but the walk's own exit tests and DDA arithmetic happens there,
@@ -338,16 +301,8 @@ __device__ __forceinline__ bool replayStep(Replay& r, int GX, int GY, int GZ, co
         if ((q1 & q2 & kGuard) == kGuard) break;                               // inside: the next call looks at the hits
         ++r.steps;
         if ((~q2 & r.gpos) | (~q1 & gneg)) finished = true;                     // passed for good (this voxel is visited, the walk ends after it)
-        else if (r.inter && (abs(r.cx - r.ix) > 2 || abs(r.cy - r.iy) > 2 || abs(r.cz - r.iz) > 2)) finished = true;
-        else {
-            const bool px = r.gpos & (1u << 9), py = r.gpos & (1u << 19), pz = r.gpos & (1u << 29);
-            const bool sx = r.tmx < r.tmy && r.tmx < r.tmz, sy = !sx && r.tmy < r.tmz;
-            r.ix += sx ? (px ? 1 : -1) : 0; r.iy += sy ? (py ? 1 : -1) : 0; r.iz += (sx || sy) ? 0 : (pz ? 1 : -1);
-            const float tsel = sx ? r.tmx : sy ? r.tmy : r.tmz;
-            const int isel = sx ? r.ix : sy ? r.iy : r.iz, lim = sx ? (px ? GX : -1) : sy ? (py ? GY : -1) : (pz ? GZ : -1);
-            if (isel == lim || tsel >= kFloatMax) finished = true;
-            else { r.tmx = sx ? xadd(r.tmx, r.dx) : r.tmx; r.tmy = sy ? xadd(r.tmy, r.dy) : r.tmy; r.tmz = (sx || sy) ? r.tmz : xadd(r.tmz, r.dz); }
-        }
+        else if (pastLastHit(r)) finished = true;
+        else finished = ddaStep(r, GX, GY, GZ);
         ++r.k;
     }
     return finished;
@@ -390,7 +345,7 @@ __device__ __forceinline__ bool replayEnter(const InstanceTrace* __restrict__ in
 __device__ __forceinline__ void replayLoadHits(const SceneDev& sc, const EmuBuf& emu, int i, int nh, int first_id, float t_star, unsigned& ulo, unsigned& uhi,
                                                unsigned* s_lo, unsigned* s_hi, float* s_ts, int* s_ids, int stride)
 {
-    ulo = 0x1ffu | (0x1ffu << 10) | (0x1ffu << 20); uhi = 0u;
+    ulo = kEmptyLo; uhi = kEmptyHi;
 #pragma unroll 1
     for (int j = 0; j < nh; ++j) {
         const int slot = j * stride + threadIdx.x;
@@ -399,10 +354,7 @@ __device__ __forceinline__ void replayLoadHits(const SceneDev& sc, const EmuBuf&
         const int2 bx = __ldg(&sc.tri_box[idj]);
         const unsigned lj = (unsigned)bx.x, hj = (unsigned)bx.y;
         s_lo[slot] = lj; s_hi[slot] = hj;
-        if ((((hj | kGuard) - lj) & kGuard) == kGuard) {                // listed somewhere (lo <= hi on every axis)
-            ulo = min(ulo & 0x1ffu, lj & 0x1ffu) | min(ulo & (0x1ffu << 10), lj & (0x1ffu << 10)) | min(ulo & (0x1ffu << 20), lj & (0x1ffu << 20));
-            uhi = max(uhi & 0x1ffu, hj & 0x1ffu) | max(uhi & (0x1ffu << 10), hj & (0x1ffu << 10)) | max(uhi & (0x1ffu << 20), hj & (0x1ffu << 20));
-        }
+        unionBox(ulo, uhi, lj, hj);
     }
 }
 
@@ -414,16 +366,7 @@ __device__ __forceinline__ void replayFinish(const SceneDev& sc, const Replay& r
     if (r.w_tri >= 0 && r.w_t == r.t_star) {
         // the walk of the nearest model finds the closest hit: that is the reference's answer (the triangle is the WALK's: its tie rule)
         if (r.w_tri != __float_as_int(h.y)) hit[r.i] = make_float4(h.x, __int_as_float(r.w_tri), h.z, h.w);
-        if (UV && uv) {                                                          // barycentrics as the predicate computes them (Renderer.cpp:174-201)
-            const InstanceTrace* __restrict__ inst = &sc.inst[__float_as_int(h.z)];
-            const float4 w0 = ldg4(&inst->w2m[0]), w1 = ldg4(&inst->w2m[1]), w2 = ldg4(&inst->w2m[2]);
-            const V3 ro = xmat4(w0, w1, w2, v3(O[r.i]), 1.0f), rd = xnormalize(xmat4(w0, w1, w2, v3(D[r.i]), 0.0f));
-            const float4 a = ldg4(&sc.tris[r.w_tri].v0), b = ldg4(&sc.tris[r.w_tri].e1), c = ldg4(&sc.tris[r.w_tri].e2);
-            const V3 pvec = xcross(rd, v3(c));
-            const float invDet = xdiv(1.0f, xdot(v3(b), pvec));
-            const V3 tvec = xsub(ro, v3(a));
-            uv[r.i] = make_float2(xmul(xdot(tvec, pvec), invDet), xmul(xdot(rd, xcross(tvec, v3(b))), invDet));
-        }
+        if (UV && uv) uv[r.i] = hitBarycentrics(sc, __float_as_int(h.z), v3(O[r.i]), v3(D[r.i]), r.w_tri);
     } else emu.list[atomicAdd(&st->n_replay[round], 1u)] = r.i;                 // the walk itself answers this one (last launch)
 }
 
@@ -476,11 +419,7 @@ k_emu_setup(SceneDev sc, const float4* __restrict__ O, const float4* __restrict_
         if (COUNT) { if (counts) counts[i].y = r.steps; steps_total += r.steps; }
         replayFinish<UV>(sc, r, h, O, D, hit, uv, st, round, emu);
     }
-    if (COUNT) {
-#pragma unroll
-        for (int d = 16; d > 0; d >>= 1) steps_total += __shfl_xor_sync(0xffffffffu, steps_total, d);
-        if ((threadIdx.x & 31) == 0) atomicAdd(&st->count_cells, steps_total);
-    }
+    if (COUNT) warpTotalAdd(&st->count_cells, steps_total);
 }
 
 template <bool UV, bool COUNT>
@@ -488,10 +427,8 @@ __global__ void __launch_bounds__(kReplayBlock)
 k_emu_tail(SceneDev sc, const float4* __restrict__ O, const float4* __restrict__ D, float4* __restrict__ hit, float2* __restrict__ uv,
            int4* __restrict__ counts, FrameState* st, int round, EmuBuf emu)
 {
-    constexpr unsigned kFullMask = 0xffffffffu;
     const int n = (int)min(st->n_cont[round], (unsigned)emu.cont_cap);
     unsigned int* cursor = &st->fetch_emu[round];
-    const int lane = threadIdx.x & 31;
     const int GX = sc.gx, GY = sc.gy, GZ = sc.gz;
     __shared__ int s_ids[kEmuHits * kReplayBlock];
     __shared__ float s_ts[kEmuHits * kReplayBlock];
@@ -500,14 +437,13 @@ k_emu_tail(SceneDev sc, const float4* __restrict__ O, const float4* __restrict__
     enum : int { R_IDLE = 0, R_STEP = 1, R_DONE = 2 };
     int state = R_IDLE;
     Replay r; r.i = -1; r.nh = 0; r.steps = 0;
-    int w_next = 0, w_end = 0;
-    bool exhausted = false;
+    WarpBatch work;
 
     for (;;) {
         // ---- one voxel of every replay in progress
         if (state == R_STEP && replayStep(r, GX, GY, GZ, s_lo, s_hi, s_ts, s_ids, kReplayBlock)) state = R_DONE;
         // ---- who is where
-        const unsigned m_step = __ballot_sync(kFullMask, state == R_STEP);
+        const unsigned m_step = __ballot_sync(kFull, state == R_STEP);
         if (m_step != 0u && 32 - __popc(m_step) < sc.emu_refill) continue;      // keep stepping until enough lanes are free (or none steps)
         // ---- results of the finished replays
         if (state == R_DONE) {
@@ -516,19 +452,12 @@ k_emu_tail(SceneDev sc, const float4* __restrict__ O, const float4* __restrict__
             state = R_IDLE; r.i = -1;
         }
         // ---- the next queue entries for the free lanes
-        if (w_next >= w_end && !exhausted) {
-            unsigned b = 0;
-            if (lane == 0) b = atomicAdd(cursor, (unsigned)kReplayBatch);
-            b = __shfl_sync(kFullMask, b, 0);
-            if (b >= (unsigned)n) { exhausted = true; w_next = w_end = n; }
-            else { w_next = (int)b; w_end = min((int)b + kReplayBatch, n); }
-        }
-        const unsigned m_idle = __ballot_sync(kFullMask, state == R_IDLE);
-        if (m_step == 0u && exhausted && w_next >= w_end) break;      // nothing in progress, nothing left (every lane is idle here)
-        const int avail = w_end - w_next;
-        const int rank = __popc(m_idle & ((1u << lane) - 1u));
-        if (state == R_IDLE && rank < avail) {
-            const uint4* rec = emu.cont + (size_t)(w_next + rank) * 5;
+        work.fetch(cursor, kReplayBatch, n);
+        const unsigned m_idle = __ballot_sync(kFull, state == R_IDLE);
+        if (m_step == 0u && work.exhausted && work.w_next >= work.w_end) break;      // nothing in progress, nothing left (every lane is idle here)
+        int next;
+        if (work.claim(m_idle, state == R_IDLE, next)) {
+            const uint4* rec = emu.cont + (size_t)next * 5;
             const uint4 a = rec[0], b = rec[1], c = rec[2], d = rec[3], e = rec[4];
             r.i = (int)a.x; r.ix = a.y & 0x3ff; r.iy = (a.y >> 10) & 0x3ff; r.iz = a.y >> 20;
             r.gpos = a.z & kGuard; r.inter = a.z & 1u; r.nh = (a.z >> 1) & 0xf; r.seen = a.w; r.passed = false;
@@ -540,13 +469,9 @@ k_emu_tail(SceneDev sc, const float4* __restrict__ O, const float4* __restrict__
             replayLoadHits(sc, emu, r.i, r.nh, __float_as_int(h.y), r.t_star, r.ulo, r.uhi, s_lo, s_hi, s_ts, s_ids, kReplayBlock);
             state = R_STEP;
         }
-        w_next += min(__popc(m_idle), avail);
+        work.advance(m_idle);
     }
-    if (COUNT) {
-#pragma unroll
-        for (int d = 16; d > 0; d >>= 1) steps_total += __shfl_xor_sync(kFullMask, steps_total, d);
-        if (lane == 0) atomicAdd(&st->count_cells, steps_total);
-    }
+    if (COUNT) warpTotalAdd(&st->count_cells, steps_total);
 }
 
 // ---- launch 4: the rays the replay could not confirm, emulated in FULL -----------------------------------------------------------------
@@ -568,15 +493,12 @@ k_emu_full(SceneDev sc, const float4* __restrict__ O, const float4* __restrict__
     const int n = (int)st->n_replay[round];
     if (blockIdx.x == 0 && threadIdx.x == 0) st->rays_reemulated += (unsigned long long)n;
     unsigned int* cursor = &st->fetch_replay[round];
-    const int lane = threadIdx.x & 31;
     const int GX = sc.gx, GY = sc.gy, GZ = sc.gz;
     if (n == 0 || sc.tlas_root < 0) return;
 
-    int sp = 0;
-    __shared__ int s_stack[kEmuStack * kTraceBlock];
-    int l_stack[kBvhStack - kEmuStack];
-    auto push = [&](int v) { if (sp < kEmuStack) s_stack[sp * kTraceBlock + threadIdx.x] = v; else l_stack[sp - kEmuStack] = v; ++sp; };
-    auto pop = [&]() { --sp; return sp < kEmuStack ? s_stack[sp * kTraceBlock + threadIdx.x] : l_stack[sp - kEmuStack]; };
+    __shared__ int s_stack[kSmemStack * kTraceBlock];
+    int l_stack[kBvhStack - kSmemStack];
+    SplitStack stack(s_stack, l_stack);
     __shared__ int s_ids[kFullHits * kTraceBlock];                  // [hit][thread]: the hits of the instance being traversed
     __shared__ float s_ts[kFullHits * kTraceBlock];
     __shared__ unsigned s_lo[kFullHits * kTraceBlock], s_hi[kFullHits * kTraceBlock];
@@ -591,45 +513,26 @@ k_emu_full(SceneDev sc, const float4* __restrict__ O, const float4* __restrict__
     float tmin = 0.0f, tmax = 0.0f;
     float g_dist = kFloatMax, g_t = 0.0f;
     int g_model = -1, g_tri = -1;
-    int w_next = 0, w_end = 0;
-    bool exhausted = false;
+    WarpBatch work;
     const int vote_tri = sc.vote_tri, vote_inst = sc.vote_inst, vote_refill = sc.vote_refill;
 
     for (;;) {
         if (node >= 0) {
             int key[4], lnk[4];
-            nodeChildren(reinterpret_cast<const char*>(&sc.nodes[node]), ro, rinv, near_off, tmin, tmax, key, lnk);
-            if (key[3] != 0x7f800000) push(lnk[3]);
-            if (key[2] != 0x7f800000) push(lnk[2]);
-            if (key[1] != 0x7f800000) push(lnk[1]);
-            if (key[0] != 0x7f800000) node = lnk[0]; else node = pop();
+            nodeChildren<true>(reinterpret_cast<const char*>(&sc.nodes[node]), ro, rinv, near_off, tmin, tmax, key, lnk);
+            node = stack.descend(key, lnk);
         }
-        const unsigned code = ~(unsigned)node;
-        const unsigned state = min(code >> 29, 4u);             // 0 tri, 1 enter, 2 exit, 3 done, 4 inner
-        const bool live = state != 3u || i >= 0 || !exhausted;
-        const unsigned sum = __reduce_add_sync(kFull, live ? 1u << (6u * state) : 0u);
-        if (sum == 0u) break;
-        const int n_tri = sum & 63u, n_enter = (sum >> 6) & 63u, n_exit = (sum >> 12) & 63u, n_done = (sum >> 18) & 63u, n_inner = (sum >> 24) & 63u;
-        const bool s_tri = state == 0u, s_enter = state == 1u, s_exit = state == 2u, s_done = state == 3u;
+        const LaneVote vt = laneVote(node, i >= 0 || !work.exhausted);
+        if (vt.n_all == 0u) break;
+        const unsigned code = vt.code;
 
         // ---- one triangle of the held leaf: the reference's predicate (Renderer.cpp:174-201), every hit recorded with its voxel box
-        if (s_tri && n_tri >= min(vote_tri, n_inner)) {
-            const int k = (int)(code >> 3);
-            const F8 ta = ldg8(&sc.bvh_tris[k]), tb = ldg8(reinterpret_cast<const char*>(&sc.bvh_tris[k]) + 32);
-            const V3 v0 = v3(ta.v[0], ta.v[1], ta.v[2]), v0v1 = v3(ta.v[3], ta.v[4], ta.v[5]), v0v2 = v3(ta.v[6], ta.v[7], tb.v[0]);
-            const V3 pvec = xcross(rd, v0v2);
-            const float det = xdot(v0v1, pvec);
-            const float invDet = xdiv(1.0f, det);
-            const V3 tvec = xsub(ro, v0);
-            const float u = xmul(xdot(tvec, pvec), invDet);
-            const V3 qvec = xcross(tvec, v0v1);
-            const float v = xmul(xdot(rd, qvec), invDet);
-            const float t = xmul(xdot(v0v2, qvec), invDet);
-            const bool reject = (xabs(xsub(det, 0.0f)) < kEpsilon) | (u < (0.0f - kEpsilon)) | (u > (1.0f + kEpsilon)) |
-                                (v < (0.0f - kEpsilon)) | (xadd(u, v) > (1.0f + kEpsilon)) | (t < (0.0f - kEpsilon));
-            if (!reject) {
+        if (vt.tri && vt.n_tri >= min(vote_tri, vt.n_inner)) {
+            const TriTest h = leafTriangle(sc, (int)(code >> 3), ro, rd);
+            if (!h.reject) {
+                const float t = h.t;
                 if (nh < kFullHits + kBigHits) {
-                    const int id = __float_as_int(tb.v[1]);
+                    const int id = h.id;
                     const int2 bx = __ldg(&sc.tri_box[id]);
                     if (nh < kFullHits) {
                         const int slot = nh * kTraceBlock + threadIdx.x;
@@ -639,24 +542,20 @@ k_emu_full(SceneDev sc, const float4* __restrict__ O, const float4* __restrict__
                 ++nh;
                 if (t < c_t) c_t = t;
             }
-            if (code & 7u) node = (int)~(code + 7u); else node = pop();
+            if (code & 7u) node = (int)~(code + 7u); else node = stack.pop();
         }
         // ---- enter instance `im` (Renderer.cpp:381-384)
-        if (s_enter && n_enter >= min(vote_inst, n_inner)) {
+        if (vt.enter && vt.n_enter >= min(vote_inst, vt.n_inner)) {
             const int im = (int)(code & kIndexMask);
             const InstanceTrace* __restrict__ inst = &sc.inst[im];
-            const float4 w0 = ldg4(&inst->w2m[0]), w1 = ldg4(&inst->w2m[1]), w2 = ldg4(&inst->w2m[2]);
-            ro = xmat4(w0, w1, w2, bo, 1.0f);                                   // Renderer.cpp:381
-            rd = xnormalize(xmat4(w0, w1, w2, bd, 0.0f));                       // Renderer.cpp:382
-            rinv = v3(safeInv(rd.x), safeInv(rd.y), safeInv(rd.z));
-            near_off = nearOffsets(rd);
-            tmin = -(kEpsilon + 1e-4f); tmax = 3.0e38f;
+            enterInstance(inst, bo, bd, ro, rd, rinv, near_off);
+            tmin = kModelTmin; tmax = 3.0e38f;
             nh = 0; c_t = kFloatMax;
-            push((int)~(kExitBit | (unsigned)im));
+            stack.push((int)~(kExitBit | (unsigned)im));
             node = __float_as_int(__ldg(&inst->grid.z));
         }
         // ---- leave instance `im`: replay its walk over the hits found, then the reference's nearest-model rule (Renderer.cpp:388-398)
-        if (s_exit && n_exit >= min(vote_inst, n_inner)) {
+        if (vt.exit && vt.n_exit >= min(vote_inst, vt.n_inner)) {
             const int im = (int)(code & kIndexMask);
             if (nh > kFullHits + kBigHits) overflow = true;
             else if (nh > kFullHits) {
@@ -665,7 +564,6 @@ k_emu_full(SceneDev sc, const float4* __restrict__ O, const float4* __restrict__
                 Replay r;
                 r.i = i; r.nh = nh; r.t_star = c_t; r.w_tri = -1; r.w_t = kFloatMax; r.steps = 0;
                 if (replayEnter(&sc.inst[im], ro, rd, GX, GY, GZ, r)) {
-                    const bool px = r.gpos & (1u << 9), py = r.gpos & (1u << 19), pz = r.gpos & (1u << 29);
                     for (;;) {
                         const unsigned v = (unsigned)r.ix | ((unsigned)r.iy << 10) | ((unsigned)r.iz << 20);
                         bool any = false;
@@ -688,13 +586,7 @@ k_emu_full(SceneDev sc, const float4* __restrict__ O, const float4* __restrict__
                         }
                         if (r.w_t == r.t_star) break;
                         if (any) { r.cx = r.ix; r.cy = r.iy; r.cz = r.iz; r.inter = true; }
-                        if (r.inter && (abs(r.cx - r.ix) > 2 || abs(r.cy - r.iy) > 2 || abs(r.cz - r.iz) > 2)) break;
-                        const bool sx = r.tmx < r.tmy && r.tmx < r.tmz, sy = !sx && r.tmy < r.tmz;
-                        r.ix += sx ? (px ? 1 : -1) : 0; r.iy += sy ? (py ? 1 : -1) : 0; r.iz += (sx || sy) ? 0 : (pz ? 1 : -1);
-                        const float tsel = sx ? r.tmx : sy ? r.tmy : r.tmz;
-                        const int isel = sx ? r.ix : sy ? r.iy : r.iz, lim = sx ? (px ? GX : -1) : sy ? (py ? GY : -1) : (pz ? GZ : -1);
-                        if (isel == lim || tsel >= kFloatMax) break;
-                        r.tmx = sx ? xadd(r.tmx, r.dx) : r.tmx; r.tmy = sy ? xadd(r.tmy, r.dy) : r.tmy; r.tmz = (sx || sy) ? r.tmz : xadd(r.tmz, r.dz);
+                        if (pastLastHit(r) || ddaStep(r, GX, GY, GZ)) break;
                         ++r.k;
                     }
                     if (r.w_tri >= 0) {
@@ -707,15 +599,9 @@ k_emu_full(SceneDev sc, const float4* __restrict__ O, const float4* __restrict__
                 Replay r;
                 r.i = i; r.nh = nh; r.t_star = c_t; r.w_tri = -1; r.w_t = kFloatMax; r.steps = 0;
                 if (replayEnter(&sc.inst[im], ro, rd, GX, GY, GZ, r)) {
-                    r.ulo = 0x1ffu | (0x1ffu << 10) | (0x1ffu << 20); r.uhi = 0u;
+                    r.ulo = kEmptyLo; r.uhi = kEmptyHi;
 #pragma unroll 1
-                    for (int j = 0; j < nh; ++j) {
-                        const unsigned lj = s_lo[j * kTraceBlock + threadIdx.x], hj = s_hi[j * kTraceBlock + threadIdx.x];
-                        if ((((hj | kGuard) - lj) & kGuard) == kGuard) {
-                            r.ulo = min(r.ulo & 0x1ffu, lj & 0x1ffu) | min(r.ulo & (0x1ffu << 10), lj & (0x1ffu << 10)) | min(r.ulo & (0x1ffu << 20), lj & (0x1ffu << 20));
-                            r.uhi = max(r.uhi & 0x1ffu, hj & 0x1ffu) | max(r.uhi & (0x1ffu << 10), hj & (0x1ffu << 10)) | max(r.uhi & (0x1ffu << 20), hj & (0x1ffu << 20));
-                        }
-                    }
+                    for (int j = 0; j < nh; ++j) unionBox(r.ulo, r.uhi, s_lo[j * kTraceBlock + threadIdx.x], s_hi[j * kTraceBlock + threadIdx.x]);
 #pragma unroll 1
                     while (!replayStep(r, GX, GY, GZ, s_lo, s_hi, s_ts, s_ids, kTraceBlock)) { }
                     if (r.w_tri >= 0) {
@@ -727,44 +613,24 @@ k_emu_full(SceneDev sc, const float4* __restrict__ O, const float4* __restrict__
             nh = 0; c_t = kFloatMax;
             ro = bo; rinv = winv; near_off = wnear_off;
             tmin = sc.tmin_world; tmax = 3.0e38f;                                // no pruning by distance: a farther model may hold the answer
-            node = pop();
+            node = stack.pop();
         }
         // ---- retire finished rays, refill the lanes from the warp's batch of the list
-        if (n_done > 0 && n_done >= min(vote_refill, n_inner)) {
-            const unsigned m_done = __ballot_sync(kFull, s_done && live);
-            if (s_done && i >= 0) {
+        if (vt.n_done > 0 && vt.n_done >= min(vote_refill, vt.n_inner)) {
+            const unsigned m_done = __ballot_sync(kFull, vt.done && vt.live);
+            if (vt.done && i >= 0) {
                 if (overflow) emu.list2[atomicAdd(&st->n_walk[round], 1u)] = i;      // more hits in one model than are kept: the walk itself
                 else {
                     const bool found = g_dist < kFloatMax;
                     hit[i] = make_float4(found ? g_dist : kFloatMax, __int_as_float(found ? g_tri : -1), __int_as_float(found ? g_model : -1), found ? g_t : 0.0f);
-                    if (UV && uv) {
-                        float2 w = make_float2(0.0f, 0.0f);
-                        if (found) {                                                     // barycentrics as the predicate computes them
-                            const InstanceTrace* __restrict__ inst = &sc.inst[g_model];
-                            const float4 w0 = ldg4(&inst->w2m[0]), w1 = ldg4(&inst->w2m[1]), w2 = ldg4(&inst->w2m[2]);
-                            const V3 mo = xmat4(w0, w1, w2, bo, 1.0f), md = xnormalize(xmat4(w0, w1, w2, bd, 0.0f));
-                            const float4 a = ldg4(&sc.tris[g_tri].v0), b = ldg4(&sc.tris[g_tri].e1), c = ldg4(&sc.tris[g_tri].e2);
-                            const V3 pvec = xcross(md, v3(c));
-                            const float invDet = xdiv(1.0f, xdot(v3(b), pvec));
-                            const V3 tvec = xsub(mo, v3(a));
-                            w = make_float2(xmul(xdot(tvec, pvec), invDet), xmul(xdot(md, xcross(tvec, v3(b))), invDet));
-                        }
-                        uv[i] = w;
-                    }
+                    if (UV && uv) uv[i] = found ? hitBarycentrics(sc, g_model, bo, bd, g_tri) : make_float2(0.0f, 0.0f);
                 }
                 i = -1;
             }
-            if (w_next >= w_end && !exhausted) {
-                unsigned b = 0;
-                if (lane == 0) b = atomicAdd(cursor, (unsigned)kFullBatch);
-                b = __shfl_sync(kFull, b, 0);
-                if (b >= (unsigned)n) { exhausted = true; w_next = w_end = n; }
-                else { w_next = (int)b; w_end = min((int)b + kFullBatch, n); }
-            }
-            const int avail = w_end - w_next;
-            const int rank = __popc(m_done & ((1u << lane) - 1u));
-            if (s_done && live && rank < avail) {
-                i = __ldg(&emu.list[w_next + rank]);
+            work.fetch(cursor, kFullBatch, n);
+            int next;
+            if (work.claim(m_done, vt.done && vt.live, next)) {
+                i = __ldg(&emu.list[next]);
                 const float4 o4 = O[i], d4 = D[i];
                 bo = v3(o4); bd = v3(d4);
                 const float il = rsqrtf(bd.x * bd.x + bd.y * bd.y + bd.z * bd.z);
@@ -774,10 +640,10 @@ k_emu_full(SceneDev sc, const float4* __restrict__ O, const float4* __restrict__
                 tmin = sc.tmin_world; tmax = 3.0e38f;
                 g_dist = kFloatMax; g_model = -1; g_tri = -1; g_t = 0.0f;
                 nh = 0; c_t = kFloatMax; overflow = false;
-                sp = 0; push(kDone);
+                stack.sp = 0; stack.push(kDone);
                 node = sc.tlas_root;
             }
-            w_next += min(__popc(m_done), avail);
+            work.advance(m_done);
         }
     }
 }

@@ -70,14 +70,12 @@ k_trace_grid(SceneDev sc, const float4* __restrict__ O, const float4* __restrict
              float2* __restrict__ uv, int4* __restrict__ counts, FrameState* st, int round, int n_fixed, unsigned long long* __restrict__ stamp,
              const int* __restrict__ list)
 {
-    constexpr unsigned kFull = 0xffffffffu;
     // list != null: the last launch of PTAP_ACCEL_GRID_EMULATED - only the slots k_emu_full (trace_emu.cu) handed over are walked
     const int n = list ? (int)st->n_walk[round] : n_fixed >= 0 ? n_fixed : st->n_active[round];
     if (blockIdx.x == 0 && threadIdx.x == 0 && n_fixed < 0 && !list) st->rays_traced += (unsigned long long)n;
     if (blockIdx.x == 0 && threadIdx.x == 0 && list) st->rays_walked += (unsigned long long)n;
     if (stamp && threadIdx.x == 0) atomicMin(stamp, globalTimerNs());
     unsigned int* cursor = list ? &st->fetch_walk[round] : &st->fetch[round];
-    const int lane = threadIdx.x & 31;
     const int GX = sc.gx, GY = sc.gy, GZ = sc.gz;
     unsigned long long tot_x = 0, tot_y = 0, tot_z = 0;
     int4 cnt = make_int4(0, 0, 0, 0);
@@ -91,13 +89,12 @@ k_trace_grid(SceneDev sc, const float4* __restrict__ O, const float4* __restrict
     int ix = 0, iy = 0, iz = 0, cx = 0, cy = 0, cz = 0, vox0 = 0, ri = 0, rend = 0;
     float tmx = kFloatMax, tmy = kFloatMax, tmz = kFloatMax, dx = kFloatMax, dy = kFloatMax, dz = kFloatMax;
     float t_entry = 0.0f;
-    int w_next = 0, w_end = 0;
-    bool exhausted = false;
+    WarpBatch work;
     const int vote = sc.vote_grid;
 
     for (;;) {
         // ---- who waits for what
-        const bool live = state != G_DONE || i >= 0 || !exhausted;
+        const bool live = state != G_DONE || i >= 0 || !work.exhausted;
         const unsigned sum = __reduce_add_sync(kFull, live ? 1u << (6u * state) : 0u);
         if (sum == 0u) break;
         const int n_model = sum & 63u, n_init = (sum >> 6) & 63u, n_cell = (sum >> 12) & 63u, n_tri = (sum >> 18) & 63u, n_done = (sum >> 24) & 63u;
@@ -223,33 +220,22 @@ k_trace_grid(SceneDev sc, const float4* __restrict__ O, const float4* __restrict
                 if (COUNT) { if (counts) counts[i] = cnt; tot_x += cnt.x; tot_y += cnt.y; tot_z += cnt.z; }
                 i = -1;
             }
-            if (w_next >= w_end && !exhausted) {
-                unsigned b = 0;
-                if (lane == 0) b = atomicAdd(cursor, (unsigned)sc.batch);
-                b = __shfl_sync(kFull, b, 0);
-                if (b >= (unsigned)n) { exhausted = true; w_next = w_end = n; }
-                else { w_next = (int)b; w_end = min((int)b + sc.batch, n); }
-            }
-            const int avail = w_end - w_next;
-            const int rank = __popc(m_done & ((1u << lane) - 1u));
-            if (s_done && live && rank < avail) {
-                i = list ? __ldg(&list[w_next + rank]) : w_next + rank;
+            work.fetch(cursor, sc.batch, n);
+            int next;
+            if (work.claim(m_done, s_done && live, next)) {
+                i = list ? __ldg(&list[next]) : next;
                 bo = v3(O[i]); bd = v3(D[i]);
                 g_dist = kFloatMax; g_model = -1; g_tri = -1; g_t = 0.0f; g_u = 0.0f; g_v = 0.0f;
                 if (COUNT) cnt = make_int4(0, 0, 0, 0);
                 im = -1; flags = 0;
                 state = G_MODEL;
             }
-            w_next += min(__popc(m_done), avail);
+            work.advance(m_done);
         }
     }
     if (stamp && (threadIdx.x & 31) == 0) atomicMax(stamp + 1, globalTimerNs());
     if (COUNT) {        // counting build: per-warp totals into the frame state (never used for timing)
-#pragma unroll
-        for (int d = 16; d > 0; d >>= 1) {
-            tot_x += __shfl_xor_sync(kFull, tot_x, d); tot_y += __shfl_xor_sync(kFull, tot_y, d); tot_z += __shfl_xor_sync(kFull, tot_z, d);
-        }
-        if (lane == 0) { atomicAdd(&st->count_cells, tot_x); atomicAdd(&st->count_refs, tot_y); atomicAdd(&st->count_tris, tot_z); }
+        warpTotalAdd(&st->count_cells, tot_x); warpTotalAdd(&st->count_refs, tot_y); warpTotalAdd(&st->count_tris, tot_z);
     }
 }
 

@@ -1,10 +1,10 @@
 #!/bin/bash
 # Builds variant libraries next to the default one, for A/B measurements on the GPU box (select with PTAP_LIB=<path>):
-#   pathtracerap_b200/variants/libptap_w8.so    PTAP_BVH_WIDTH=8: eight children per node, IEEE-half offsets
-# usage: tools/build_variants.sh [name=flags ...]      e.g.  tools/build_variants.sh w8=-DPTAP_BVH_WIDTH=8
+#   pathtracerap_b200/variants/libptap_ctas7.so    PTAP_TRACE_MIN_CTAS=7: k_trace_bvh compiled for 7 resident CTAs per SM instead of 8
+# usage: tools/build_variants.sh [name=flags ...]      e.g.  tools/build_variants.sh ctas7=-DPTAP_TRACE_MIN_CTAS=7
 set -euo pipefail
 ROOT="$(cd "$(dirname "$0")/.." && pwd)"
-[ $# -gt 0 ] || set -- "w8=-DPTAP_BVH_WIDTH=8"
+[ $# -gt 0 ] || set -- "ctas7=-DPTAP_TRACE_MIN_CTAS=7"
 mkdir -p "$ROOT/pathtracerap_b200/variants"
 for spec in "$@"; do
   name="${spec%%=*}"; flags="${spec#*=}"
