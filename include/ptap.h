@@ -172,7 +172,10 @@ int ptap_scene_add_icosphere(ptap_scene* s, int32_t level, float radius, float d
 int ptap_scene_add_model(ptap_scene* s, int32_t mesh_index, const float model_to_world[16], const float* world_to_model, const PtapMaterial* mat, int32_t* model_index);
 /* glm::translate * glm::rotate(Y) * glm::scale as every model of Scene.cpp composes it; writes model_to_world, world_to_model */
 void ptap_compose_trs(const float translate[3], float rotate_y_degrees, const float scale[3], float model_to_world[16], float world_to_model[16]);
-/* Scene::addMeshesToGrid (Scene.cpp:318-396) */
+/* Scene::addMeshesToGrid (Scene.cpp:318-396).  Limits: gx, gy, gz >= 1 and at most 2^27 cells per grid, at most 2^31 - 1 cells over all
+ * grids (one per distinct mesh) and at most 2^31 - 1 references in all (voxels and reference positions are 32-bit).  PTAP_E_INVALID
+ * otherwise, with the count in ptap_scene_last_error; the scene keeps its previous grids.  The GRID key of a Config.txt takes the same
+ * dimensions (PTAP_E_PARSE for bad ones). */
 int ptap_scene_build_grids(ptap_scene* s, int32_t gx, int32_t gy, int32_t gz);
 /* Builds one BVH per mesh on the host (binned SAH); part of scene construction like addMeshesToGrid, so that
  * Renderer::allocateOnGPU only uploads.  Bounds are conservative for the reference's tolerance band (DESIGN.md). */
@@ -205,7 +208,8 @@ enum { PTAP_ACCEL_GRID_COMPAT = 0,  /* the reference's per-mesh uniform grid wal
                                        over the voxel boxes of the hit triangles (trace_emu.cu).  Needs the grids (their lists define the
                                        result) and builds a BVH on the device if none is there.  ptap_build_accel fails with
                                        PTAP_E_UNSUPPORTED when the lists on the device do not have the shape Scene::addMeshesToGrid
-                                       produces (Scene.cpp:357-374); PTAP_ACCEL_GRID_COMPAT then remains available. */
+                                       produces (Scene.cpp:357-374), or when an axis has more than 512 voxels (the packed voxel
+                                       index has 9 bits per axis); PTAP_ACCEL_GRID_COMPAT then remains available. */
 
 enum { PTAP_FLAG_FIRST_HIT_CACHE = 1,   /* Renderer.cpp:580,594-613 */
        PTAP_FLAG_PROFILE = 2,           /* per-kernel CUDA-event split in PtapStats (adds event records) */
@@ -236,7 +240,9 @@ int ptap_update_models(ptap_ctx* ctx, const PtapModel* models, int32_t first, in
  * triangles are read again): one gx x gy x gz grid per distinct mesh in model order, built by sorting (cell, triangle) pairs; cells and
  * reference lists are bit-identical to the host builder's / the reference's (ascending triangle order per cell).  Selects
  * PTAP_ACCEL_GRID_COMPAT; PtapStats::ms_build reports the device time.  ptap_read_grids copies the result back in the reference's layout
- * (voxels / refs NULL: counts only; counts = {voxels, references}). */
+ * (voxels / refs NULL: counts only; counts = {voxels, references}).  The limits of ptap_scene_build_grids apply: PTAP_E_INVALID, with the
+ * count in ptap_last_error, for more than 2^27 cells per grid, 2^31 - 1 cells over all grids or 2^31 - 1 references; the context then
+ * keeps its grids and accel. */
 int ptap_build_grids_device(ptap_ctx* ctx, const PtapSceneView* view, int32_t gx, int32_t gy, int32_t gz);
 int ptap_read_grids(ptap_ctx* ctx, PtapVoxel* voxels, int32_t* refs, int32_t counts[2]);
 int ptap_set_render_params(ptap_ctx* ctx, int32_t W, int32_t H, int32_t depth, uint32_t flags);

@@ -820,6 +820,9 @@ int ptap_build_accel(ptap_ctx* ctx, int kind)
         // the walk's results through the BVH (trace_emu.cu): needs the grids (their lists define the result), a BVH over the same triangles
         // (whichever builder made the one on the device; else the device builder), and lists of the shape the emulation relies on
         if (!ctx->have_grid) return fail(ctx, PTAP_E_STATE, "build_accel: the uploaded scene carries no grids (call ptap_scene_build_grids first)");
+        if (ctx->sc.gx > 512 || ctx->sc.gy > 512 || ctx->sc.gz > 512)        // 9 bits per axis in the packed voxel index (trace_emu.cu)
+            return fail(ctx, PTAP_E_UNSUPPORTED, "build_accel: the emulated walk takes at most 512 voxels per axis, the grid is %dx%dx%d; use PTAP_ACCEL_GRID_COMPAT",
+                        ctx->sc.gx, ctx->sc.gy, ctx->sc.gz);
         if (!ctx->have_bvh) { const int rc = buildBvhOnDevice(ctx); if (rc) return rc; }
         if (!ctx->emu_ok) {
             const int nt = ctx->ntris, ng = (int)ctx->h_grid_first.size();
@@ -1591,7 +1594,7 @@ int ptap_reduce(ptap_ctx* ctx, int32_t root)
 int ptap_build_grids_device(ptap_ctx* ctx, const PtapSceneView* v, int32_t gx, int32_t gy, int32_t gz)
 {
     if (!ctx || !ctx->have_scene || !v || !v->vertices || !v->triangles || !v->meshes || !v->models) return fail(ctx, PTAP_E_STATE, "build_grids_device: uploaded scene and its view required");
-    if (gx <= 0 || gy <= 0 || gz <= 0 || (long long)gx * gy * gz > (1ll << 27)) return fail(ctx, PTAP_E_INVALID, "build_grids_device: bad grid dimensions");
+    if (!gridDimsOk(gx, gy, gz)) return fail(ctx, PTAP_E_INVALID, "build_grids_device: bad grid dimensions");
     if (v->ntriangles != ctx->ntris || v->nmodels != (int)ctx->h_models.size() || v->nmeshes != (int)ctx->h_meshes.size()) return fail(ctx, PTAP_E_INVALID, "build_grids_device: the view is not the uploaded scene");
     if (const int rc = enter(ctx)) return rc;
     BuildTimer timer{ctx};
@@ -1608,6 +1611,8 @@ int ptap_build_grids_device(ptap_ctx* ctx, const PtapSceneView* v, int32_t gx, i
         model_grid[i] = grid_of_mesh[mi];
     }
     const int ng = (int)grid_mesh.size();
+    if ((long long)ng * (long long)ncell > INT32_MAX)        // k_trace_grid and the instance records index cells with int
+        return fail(ctx, PTAP_E_INVALID, "build_grids_device: %d grids x %zu cells = %lld cells exceed 2^31 - 1", ng, ncell, (long long)ng * (long long)ncell);
     // vertex positions per triangle (9 floats), gathered on the host once
     std::vector<float> pos((size_t)nt * 9);
     for (int t = 0; t < nt; ++t)
@@ -1619,11 +1624,12 @@ int ptap_build_grids_device(ptap_ctx* ctx, const PtapSceneView* v, int32_t gx, i
     int max_tris = 1;
     for (int g = 0; g < ng; ++g) max_tris = std::max(max_tris, v->meshes[grid_mesh[g]].t_end - v->meshes[grid_mesh[g]].t_start);
     // phase 1: count the references of every grid
-    DevMem<float> d_pos; DevMem<int> d_count, d_offset_all; DevMem<void> d_tmp;
+    DevMem<float> d_pos; DevMem<int> d_count, d_offset_all; DevMem<long long> d_sum; DevMem<void> d_tmp;
     size_t tmp_bytes = gridDeviceTempBytes(max_tris, 1);
     CK(cudaMalloc(d_pos.put(), pos.size() * sizeof(float) + 16));
     CK(cudaMalloc(d_count.put(), (size_t)max_tris * sizeof(int)));
     CK(cudaMalloc(d_offset_all.put(), (size_t)std::max(nt, 1) * sizeof(int)));
+    CK(cudaMalloc(d_sum.put(), sizeof(long long)));
     CK(cudaMalloc(d_tmp.put(), tmp_bytes));
     CK(cudaMemcpyAsync(d_pos, pos.data(), pos.size() * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
     std::vector<long long> npairs(ng, 0);
@@ -1634,10 +1640,11 @@ int ptap_build_grids_device(ptap_ctx* ctx, const PtapSceneView* v, int32_t gx, i
         for (int k = 0; k < 3; ++k) widths[g][k] = (mesh.bb_max[k] - mesh.bb_min[k]) / gd[k];      // Scene.cpp:341-347
         const int n = std::max(0, mesh.t_end - mesh.t_start);
         CK((cudaError_t)gridDeviceCount(d_pos + (size_t)mesh.t_start * 9, mesh.t_start, n, mesh.bb_min, widths[g].data(), gd, d_count, d_offset_all + mesh.t_start,
-                                        d_tmp, tmp_bytes, ctx->stream, &npairs[g]));
+                                        d_sum, d_tmp, tmp_bytes, ctx->stream, &npairs[g]));
         total += npairs[g]; max_pairs = std::max(max_pairs, npairs[g]);
+        // the reference list and the positions into it are 32-bit; refused here, the context keeps its grids
+        if (total > INT32_MAX) return fail(ctx, PTAP_E_INVALID, "build_grids_device: %lld references (grid %d: %lld) exceed 2^31 - 1", total, g, npairs[g]);
     }
-    if (total > 0x7fffffffll) return fail(ctx, PTAP_E_NOMEM, "build_grids_device: %lld references exceed the 32-bit reference list", total);
     // phase 2: pairs, sort, cells
     ctx->gd_cells.reset(); ctx->gd_refs.reset(); d_tmp.reset();
     tmp_bytes = gridDeviceTempBytes(max_tris, max_pairs);

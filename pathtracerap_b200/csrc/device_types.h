@@ -15,6 +15,14 @@ constexpr int kBigHits = 108;               // k_emu_full: further hits of a (ra
 constexpr int kEmuHits = 8;                 // PTAP_ACCEL_GRID_EMULATED: hits of a (ray, model) that are kept for the replay of the walk
 constexpr int kBvhStack = 160;              // traversal stack entries per ray (upload fails for deeper trees)
 
+// Grid dimensions both grid builders and Config.txt's GRID accept: every axis >= 1, at most 2^27 cells.  The product is formed in two
+// steps so that it cannot overflow: gx * gy < 2^62, and once that is <= 2^27, times gz < 2^58.
+constexpr long long kMaxGridCells = 1ll << 27;
+inline bool gridDimsOk(long long gx, long long gy, long long gz)
+{
+    return gx >= 1 && gy >= 1 && gz >= 1 && gx <= kMaxGridCells && gy <= kMaxGridCells && gx * gy <= kMaxGridCells && gx * gy * gz <= kMaxGridCells;
+}
+
 // Per-model record read by the closest-hit kernels: 9 x float4 = 144 B.
 // Rows 0..2 of the reference's column-major mat4s (the w row is never used by
 // transformPosition/transformDirection, utility.h:71-80).

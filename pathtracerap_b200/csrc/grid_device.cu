@@ -4,7 +4,7 @@
 //
 //   1  k_grid_ranges  per triangle: the voxel range it covers, with the reference's own arithmetic - floor(abs(bbox.min - tri.{min,max}) /
 //                     width) clamped to the grid (Scene.cpp:300-315), every operation an IEEE binary32 one - and the number of cells
-//   2  exclusive scan of the counts (cub)                                                    [library call, off the render path]
+//   2  sum of the counts in 64 bits, then their exclusive scan in 32 (cub)                    [library call, off the render path]
 //   3  k_grid_pairs   per triangle: one (cell, triangle) pair per covered cell, written at the triangle's offset; triangles are
 //                     processed in ascending order, so the pair list is ordered by triangle
 //   4  stable radix sort of the pairs by cell (cub): inside a cell the triangles stay ascending, exactly the order the reference's
@@ -13,7 +13,9 @@
 // The output (cells, reference list) is bit-identical to the host builder's (scene_host.cpp: buildGrids), which tests/test_host.py pins to
 // the reference's own output.
 #include <cub/device/device_radix_sort.cuh>
+#include <cub/device/device_reduce.cuh>
 #include <cub/device/device_scan.cuh>
+#include <thrust/iterator/transform_iterator.h>
 
 #include "kernels.cuh"
 
@@ -63,15 +65,19 @@ __global__ void k_grid_cells(const int* __restrict__ keys, int npairs, int ncell
 {
     const int c = blockIdx.x * blockDim.x + threadIdx.x;
     if (c >= ncell) return;
-    auto lower = [&](int key) { int a = 0, b = npairs; while (a < b) { const int m = (a + b) >> 1; if (keys[m] < key) a = m + 1; else b = m; } return a; };
+    auto lower = [&](int key) { int a = 0, b = npairs; while (a < b) { const int m = a + ((b - a) >> 1); if (keys[m] < key) a = m + 1; else b = m; } return a; };
     cells[c] = make_int2(ref_base + lower(c), ref_base + lower(c + 1));
 }
 
+struct Widen { __host__ __device__ long long operator()(int x) const { return x; } };
+using WideCounts = thrust::transform_iterator<Widen, const int*, long long>;
+
 }  // namespace
 
-// Counts the references of one mesh's grid: *npairs (synchronises the stream).  d_count / d_offset: n ints each.
+// Counts the references of one mesh's grid: *npairs, summed in 64 bits (synchronises the stream).  d_count / d_offset: n ints each,
+// d_sum: one long long.  The offsets are scanned only when *npairs fits an int; above INT32_MAX the caller refuses the mesh.
 int gridDeviceCount(const float* d_pos, int t0, int n, const float bb_min[3], const float width[3], const int gd[3], int* d_count, int* d_offset,
-                    void* d_tmp, size_t tmp_bytes, cudaStream_t stream, long long* npairs)
+                    long long* d_sum, void* d_tmp, size_t tmp_bytes, cudaStream_t stream, long long* npairs)
 {
     GridParams g;
     for (int k = 0; k < 3; ++k) { g.bb_min[k] = bb_min[k]; g.width[k] = width[k]; g.gd[k] = gd[k]; }
@@ -79,14 +85,12 @@ int gridDeviceCount(const float* d_pos, int t0, int n, const float bb_min[3], co
     *npairs = 0;
     if (n <= 0) return cudaSuccess;
     k_grid_ranges<<<(n + 255) / 256, 256, 0, stream>>>(d_pos, g, d_count);
-    cudaError_t e = cub::DeviceScan::ExclusiveSum(d_tmp, tmp_bytes, d_count, d_offset, n, stream);
-    if (e != cudaSuccess) return e;
-    int last_off = 0, last_cnt = 0;
-    e = cudaMemcpyAsync(&last_off, d_offset + n - 1, sizeof(int), cudaMemcpyDeviceToHost, stream);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(&last_cnt, d_count + n - 1, sizeof(int), cudaMemcpyDeviceToHost, stream);
+    cudaError_t e = cub::DeviceReduce::Sum(d_tmp, tmp_bytes, WideCounts((const int*)d_count, Widen()), d_sum, n, stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(npairs, d_sum, sizeof(long long), cudaMemcpyDeviceToHost, stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(stream);
     if (e != cudaSuccess) return e;
-    *npairs = (long long)last_off + last_cnt;
+    if (*npairs <= INT32_MAX) e = cub::DeviceScan::ExclusiveSum(d_tmp, tmp_bytes, d_count, d_offset, n, stream);
+    if (e != cudaSuccess) return e;
     return cudaGetLastError();
 }
 
@@ -191,10 +195,11 @@ int gridTriBoxes(const int2* cells, const int* refs, int ngrids, const int* grid
 
 size_t gridDeviceTempBytes(int ntris, long long npairs)
 {
-    size_t a = 0, b = 0;
+    size_t a = 0, b = 0, c = 0;
     cub::DeviceScan::ExclusiveSum(nullptr, a, (const int*)nullptr, (int*)nullptr, std::max(ntris, 1));
     cub::DeviceRadixSort::SortPairs(nullptr, b, (const int*)nullptr, (int*)nullptr, (const int*)nullptr, (int*)nullptr, (int)std::max(npairs, 1ll), 0, 30);
-    return std::max(a, b) + 256;
+    cub::DeviceReduce::Sum(nullptr, c, WideCounts((const int*)nullptr, Widen()), (long long*)nullptr, std::max(ntris, 1));
+    return std::max(std::max(a, b), c) + 256;
 }
 
 }  // namespace ptap

@@ -120,7 +120,7 @@ int updateInstancesDevice(InstanceTrace* inst, InstanceShade* shade, int nmodels
 
 // grid_device.cu: Scene::addMeshesToGrid on the device, one mesh's grid at a time
 int gridDeviceCount(const float* d_pos, int t0, int n, const float bb_min[3], const float width[3], const int gd[3], int* d_count, int* d_offset,
-                    void* d_tmp, size_t tmp_bytes, cudaStream_t stream, long long* npairs);
+                    long long* d_sum, void* d_tmp, size_t tmp_bytes, cudaStream_t stream, long long* npairs);
 int gridDeviceFill(const float* d_pos, int t0, int n, const float bb_min[3], const float width[3], const int gd[3], const int* d_offset, int npairs,
                    int* d_keys, int* d_vals, int* d_keys2, void* d_tmp, size_t tmp_bytes, int ref_base, int* d_refs, int2* d_cells, cudaStream_t stream);
 size_t gridDeviceTempBytes(int ntris, long long npairs);

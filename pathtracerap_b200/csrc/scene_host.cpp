@@ -7,6 +7,8 @@
 // the Config.txt schema the reference only sketched, synthetic meshes for the large-scene configs, and a counting
 // (two-pass, CSR) grid build instead of vector<vector<int>>.
 #include <algorithm>
+#include <array>
+#include <climits>
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
@@ -337,25 +339,25 @@ int addIcosphere(ptap_scene* s, int level, float radius, float displacement, uin
 int f2iX86(float x) { return (x >= -2147483648.0f && x < 2147483648.0f) ? (int)x : (-2147483647 - 1); }
 int clampi(int v, int lo, int hi) { return v < lo ? lo : (v > hi ? hi : v); }
 
-void buildGrids(ptap_scene* s, int gx, int gy, int gz)
+// Fails (PTAP_E_INVALID, s->err names the count, the scene's previous grids kept) when the grids would hold more than 2^31 - 1 cells or
+// references in all: voxels and reference positions are 32-bit.  Both counts are taken before any per-cell work.
+int buildGrids(ptap_scene* s, int gx, int gy, int gz)
 {
-    s->grid_dim[0] = gx; s->grid_dim[1] = gy; s->grid_dim[2] = gz;
-    s->grids.clear(); s->voxels.clear(); s->refs.clear();
     const int gd[3] = {gx, gy, gz};
     const size_t ncell = (size_t)gx * gy * gz;
-    std::vector<int> grid_of_mesh(s->meshes.size(), -1);
+    // grid list (Scene.cpp:322-339) and every listed triangle's voxel index box
+    std::vector<int> grid_of_mesh(s->meshes.size(), -1), grid_model;
+    std::vector<std::array<float, 3>> widths;
+    std::vector<std::vector<int>> lohis;
+    long long total = 0;
     for (size_t i = 0; i < s->models.size(); ++i) {
-        PtapModel& model = s->models[i];
-        const int mi = model.mesh_index;
-        if (grid_of_mesh[mi] >= 0) { model.grid_index = grid_of_mesh[mi]; continue; }     // Scene.cpp:325-329
-        grid_of_mesh[mi] = (int)s->grids.size();
-        model.grid_index = (int)s->grids.size();
+        const int mi = s->models[i].mesh_index;
+        if (grid_of_mesh[mi] >= 0) continue;                                                // Scene.cpp:325-329
+        grid_of_mesh[mi] = (int)grid_model.size();
+        grid_model.push_back((int)i);
         const PtapMesh& mesh = s->meshes[mi];
-        PtapGrid g{};
-        g.entity_type = 0;                  // EntityType::MODEL
-        g.entity_index = (int)i;            // the creating model: the traversal reads the bbox through it (Renderer.cpp:245-249)
-        for (int k = 0; k < 3; ++k) g.width[k] = (mesh.bb_max[k] - mesh.bb_min[k]) / gd[k];   // Scene.cpp:341-347
-        std::vector<int> offs(ncell + 1, 0), cursor;
+        std::array<float, 3> w;
+        for (int k = 0; k < 3; ++k) w[k] = (mesh.bb_max[k] - mesh.bb_min[k]) / gd[k];   // Scene.cpp:341-347
         std::vector<int> lohi((size_t)std::max(0, mesh.t_end - mesh.t_start) * 6);
         for (int t = mesh.t_start; t < mesh.t_end; ++t) {
             float tmn[3] = {kFloatMax, kFloatMax, kFloatMax}, tmx[3] = {kFloatMin, kFloatMin, kFloatMin};
@@ -365,9 +367,31 @@ void buildGrids(ptap_scene* s, int gx, int gy, int gz)
             }
             int* lh = &lohi[(size_t)(t - mesh.t_start) * 6];
             for (int k = 0; k < 3; ++k) {    // floor(abs(bbox.min - tri.{min,max}) / width) clamped (Scene.cpp:300-315)
-                lh[k] = clampi(f2iX86(std::floor(std::fabs(mesh.bb_min[k] - tmn[k]) / g.width[k])), 0, gd[k] - 1);
-                lh[3 + k] = clampi(f2iX86(std::floor(std::fabs(mesh.bb_min[k] - tmx[k]) / g.width[k])), 0, gd[k] - 1);
+                lh[k] = clampi(f2iX86(std::floor(std::fabs(mesh.bb_min[k] - tmn[k]) / w[k])), 0, gd[k] - 1);
+                lh[3 + k] = clampi(f2iX86(std::floor(std::fabs(mesh.bb_min[k] - tmx[k]) / w[k])), 0, gd[k] - 1);
             }
+            total += (long long)(lh[3] - lh[0] + 1) * (lh[4] - lh[1] + 1) * (lh[5] - lh[2] + 1);
+        }
+        widths.push_back(w);
+        lohis.push_back(std::move(lohi));
+    }
+    const long long cells = (long long)grid_model.size() * (long long)ncell;
+    if (cells > INT32_MAX) { s->err = "build_grids: " + std::to_string(grid_model.size()) + " grids x " + std::to_string(ncell) + " cells = " + std::to_string(cells) + " cells exceed 2^31 - 1"; return PTAP_E_INVALID; }
+    if (total > INT32_MAX) { s->err = "build_grids: " + std::to_string(total) + " references exceed 2^31 - 1"; return PTAP_E_INVALID; }
+    s->grid_dim[0] = gx; s->grid_dim[1] = gy; s->grid_dim[2] = gz;
+    s->grids.clear(); s->voxels.clear(); s->refs.clear();
+    s->voxels.reserve((size_t)cells); s->refs.reserve((size_t)total);
+    for (size_t i = 0; i < s->models.size(); ++i) s->models[i].grid_index = grid_of_mesh[s->models[i].mesh_index];
+    for (size_t gi = 0; gi < grid_model.size(); ++gi) {
+        const PtapMesh& mesh = s->meshes[s->models[grid_model[gi]].mesh_index];
+        PtapGrid g{};
+        g.entity_type = 0;                  // EntityType::MODEL
+        g.entity_index = grid_model[gi];    // the creating model: the traversal reads the bbox through it (Renderer.cpp:245-249)
+        for (int k = 0; k < 3; ++k) g.width[k] = widths[gi][k];
+        std::vector<int> offs(ncell + 1, 0), cursor;
+        const std::vector<int>& lohi = lohis[gi];
+        for (int t = mesh.t_start; t < mesh.t_end; ++t) {
+            const int* lh = &lohi[(size_t)(t - mesh.t_start) * 6];
             for (int z = lh[2]; z <= lh[5]; ++z)
                 for (int y = lh[1]; y <= lh[4]; ++y)
                     for (int x = lh[0]; x <= lh[3]; ++x) offs[(size_t)x + (size_t)y * gx + (size_t)gx * gy * z + 1]++;
@@ -390,6 +414,7 @@ void buildGrids(ptap_scene* s, int gx, int gy, int gz)
         g.v_end = (int)s->voxels.size();
         s->grids.push_back(g);
     }
+    return PTAP_OK;
 }
 
 // ---- the scene hard-coded in Scene::Scene (Scene.cpp:3-224): data, not algorithm ---------------------------------
@@ -520,7 +545,14 @@ int parseConfig(ptap_scene* s, const std::string& path)
                 if (i + 1 >= b.size()) { s->err = path + ": " + up + " needs a value"; return PTAP_E_PARSE; }
                 float v[3] = {0, 0, 0};
                 if (up == "RESOLUTION") { if (!parseVec(b[i + 1], v, 2)) { s->err = path + ": bad RESOLUTION"; return PTAP_E_PARSE; } s->cfg_width = (int)v[0]; s->cfg_height = (int)v[1]; }
-                else if (up == "GRID") { if (!parseVec(b[i + 1], v, 3)) { s->err = path + ": bad GRID"; return PTAP_E_PARSE; } for (int k = 0; k < 3; ++k) s->grid_dim[k] = (int)v[k]; }
+                else if (up == "GRID") {
+                    // each dimension in [1, 2^27] as a float before the conversion ((int) of an out-of-range float is undefined), then the
+                    // limits of ptap_scene_build_grids
+                    bool ok = parseVec(b[i + 1], v, 3);
+                    for (int k = 0; k < 3; ++k) ok = ok && v[k] >= 1.0f && v[k] <= (float)ptap::kMaxGridCells;
+                    if (!ok || !ptap::gridDimsOk((int)v[0], (int)v[1], (int)v[2])) { s->err = path + ": bad GRID"; return PTAP_E_PARSE; }
+                    for (int k = 0; k < 3; ++k) s->grid_dim[k] = (int)v[k];
+                }
                 else if (up == "ITER") s->cfg_iter = atoi(b[i + 1].c_str());
                 else s->cfg_depth = atoi(b[i + 1].c_str());
                 i += 2; continue;
@@ -585,8 +617,7 @@ int parseConfig(ptap_scene* s, const std::string& path)
         s->models.push_back(m);
     }
     if (s->models.empty()) { s->err = path + ": no objects"; return PTAP_E_PARSE; }
-    buildGrids(s, s->grid_dim[0], s->grid_dim[1], s->grid_dim[2]);
-    return PTAP_OK;
+    return buildGrids(s, s->grid_dim[0], s->grid_dim[1], s->grid_dim[2]);
 }
 
 }  // namespace
@@ -651,9 +682,9 @@ int ptap_scene_add_model(ptap_scene* s, int32_t mesh_index, const float model_to
 
 int ptap_scene_build_grids(ptap_scene* s, int32_t gx, int32_t gy, int32_t gz)
 {
-    if (!s || gx <= 0 || gy <= 0 || gz <= 0 || (long long)gx * gy * gz > (1ll << 27)) return PTAP_E_INVALID;
-    buildGrids(s, gx, gy, gz);
-    return PTAP_OK;
+    if (!s) return PTAP_E_INVALID;
+    if (!ptap::gridDimsOk(gx, gy, gz)) { s->err = "build_grids: bad grid dimensions"; return PTAP_E_INVALID; }
+    return buildGrids(s, gx, gy, gz);
 }
 
 int ptap_scene_create_builtin(const char* root, ptap_scene** out)
@@ -674,7 +705,7 @@ int ptap_scene_create_builtin(const char* root, ptap_scene** out)
         m.mat.type = b.type; memcpy(m.mat.color, b.color, 12);
         s->models.push_back(m);
     }
-    buildGrids(s, 25, 25, 25);                                   // Config.h:8-10, Scene.cpp:223
+    if (const int rc = buildGrids(s, 25, 25, 25)) { delete s; return rc; }      // Config.h:8-10, Scene.cpp:223
     *out = s;
     return PTAP_OK;
 }

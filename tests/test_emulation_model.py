@@ -128,6 +128,15 @@ def test_emulation_algorithm_on_the_reference_scene(port, oracle_scene, golden_t
     assert (want["model"] >= 0).mean() > 0.5
 
 
+@pytest.mark.parametrize("shape", [(7, 40, 3), (64, 1, 3)], ids=lambda s: "x".join(map(str, s)))
+def test_emulation_algorithm_on_non_cubic_grids(port, golden_scene, shape):
+    """The same algorithm on grids whose axes differ (and a thin one): voxel boxes, clamps and walk limits per axis."""
+    scene = port.OracleScene({k: golden_scene[k] for k in ("models", "meshes", "vertices", "triangles")}, grid_dim=shape)
+    routes, want = _check(scene, _rays(3000, 41))
+    assert routes["confirmed"] > 0.5 * 3000 and routes["full"] > 0
+    assert (want["model"] >= 0).mean() > 0.5
+
+
 def test_emulation_algorithm_bounce_rays(port, oracle_scene):
     """Rays that start 0.1 above a surface, as the shade kernel restarts them (Renderer.cpp:471-476): the hit just left lies inside the
     predicate's -EPSILON band behind the origin, the case fact 3's exception is about."""

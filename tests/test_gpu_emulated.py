@@ -202,28 +202,31 @@ def test_emulated_on_the_million_triangle_mesh(libptap):
     r.free()
 
 
-@pytest.mark.parametrize("dim", [25, 64])
-def test_emulated_on_a_dense_mesh(libptap, port, dim):
-    """An 82 k-triangle displaced icosphere in the room (BASELINE configs[1]) through a 25^3 and a 64^3 grid built ON THE DEVICE: hundreds
-    of triangles per voxel at 25^3, a handful at 64^3.  The emulation must equal the walk (GPU against GPU on 400 k camera + bounce rays,
-    and a whole frame), and both the oracle's R0 on a subset."""
+DENSE_SHAPES = [(25, 25, 25), (64, 64, 64), (160, 160, 160), (96, 40, 160)]
+
+
+@pytest.mark.parametrize("shape", DENSE_SHAPES, ids=[str(s[0]) if s[0] in (25, 64) else "x".join(map(str, s)) for s in DENSE_SHAPES])
+def test_emulated_on_a_dense_mesh(libptap, port, shape):
+    """An 82 k-triangle displaced icosphere in the room (BASELINE configs[1]) through grids built ON THE DEVICE: hundreds of triangles per
+    voxel at 25^3, a handful at 64^3, less than one at the benchmarked 160^3, and a grid whose axes differ.  The emulation must equal the
+    walk (GPU against GPU on 400 k camera + bounce rays, and a whole frame), and both the oracle's R0 on a subset."""
     import bench
     from pathtracerap_b200 import ACCEL_BVH, ACCEL_GRID_COMPAT, ACCEL_GRID_EMULATED, Renderer
     from test_gpu_large import _bounce_rays, _camera_rays
     scene, arrays = bench.build_scene("mesh100k")
     r = Renderer(width=64, height=32, depth=5, accel=ACCEL_BVH)        # uploaded without grids; device-built tree
     r.allocateOnGPU(scene)
-    r.build_grids_device(scene, dim, dim, dim)
+    r.build_grids_device(scene, *shape)
     cam = _camera_rays(640, 360)
     rays = np.concatenate([cam, _bounce_rays(170_000, 11)])
     walked = r.trace(rays)
     r.set_accel(ACCEL_GRID_EMULATED)
     emulated = r.trace(rays)
-    assert_hits_equal(emulated, walked, f"mesh100k {dim}^3: emulated vs walked")
+    assert_hits_equal(emulated, walked, f"mesh100k {shape}: emulated vs walked")
     assert (walked["model"] == len(arrays["models"]) - 1).mean() > 0.2
     sub = rays[:: len(rays) // 3000]
-    oscene = port.OracleScene(arrays, grid_dim=(dim, dim, dim))
-    assert_hits_equal(r.trace(sub), oscene.trace(sub, 0), f"mesh100k {dim}^3: emulated vs oracle R0")
+    oscene = port.OracleScene(arrays, grid_dim=shape)
+    assert_hits_equal(r.trace(sub), oscene.trace(sub, 0), f"mesh100k {shape}: emulated vs oracle R0")
     W, H, depth, iters = 320, 180, 5, 4
     films = []
     for accel in (ACCEL_GRID_COMPAT, ACCEL_GRID_EMULATED):

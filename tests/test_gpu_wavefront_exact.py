@@ -137,9 +137,10 @@ def _model_rounds(rounds, alb):
     return out
 
 
-def check_frame(r, alb, W, H, depth, iters, dir_iters=(0,), oracle_scene=None):
+def check_frame(r, alb, W, H, depth, iters, dir_iters=(0,), oracle_scene=None, tier=1):
     """Every round of every iteration of a frame against the model, then ptap_render's film against predict_film bit for bit.
-    Directions are compared on the iterations in dir_iters (the others add nothing the first does not); returns the probes."""
+    Directions are compared on the iterations in dir_iters (the others add nothing the first does not); with an oracle scene the first
+    iteration's hits are compared with the oracle's tier `tier` (R0: the grid walk, R1: the exact closest hit).  Returns the probes."""
     N = W * H
     probes, lengths, worst = [], [], 0.0
     for it in range(iters):
@@ -149,7 +150,7 @@ def check_frame(r, alb, W, H, depth, iters, dir_iters=(0,), oracle_scene=None):
         for k, (rays, pix, hits) in enumerate(rounds):
             what = f"{W}x{H} depth {depth} iter {it} round {k}"
             if oracle_scene is not None and it == 0:
-                _assert_production_hits(hits, oracle_scene.trace(rays, 1), what)
+                _assert_production_hits(hits, oracle_scene.trace(rays, tier), what)
             _, hit, typ, a = mr[k]
             m = sm.shade(rays[:, :3], rays[:, 3:], np.ones((len(rays), 3), np.float32), hit, hits["dist"], hits["normal"], typ, a, it,
                          depth - k, directions=it in dir_iters)

@@ -50,6 +50,133 @@ def test_grid_builder_matches_reference_golden(libptap, golden_scene):
     assert np.array_equal(a["models"]["grid_index"], g["models"]["grid_index"])
 
 
+# Grid shapes on which every stride or limit swapped between two axes changes a result: pairwise distinct dimensions none of which
+# divides another, thin grids, a power-of-two cell count (the device builder's radix-sort bit count), the benchmarked 160^3, and the
+# emulated walk's 512-per-axis limit from both sides.
+GRID_SHAPES = [(7, 40, 3), (40, 3, 7), (3, 7, 40), (1, 1, 1), (1, 64, 1), (64, 1, 3), (16, 16, 16), (160, 160, 160), (512, 4, 9), (513, 4, 9)]
+
+
+@pytest.mark.parametrize("shape", GRID_SHAPES, ids=lambda s: "x".join(map(str, s)))
+def test_grid_builder_matches_oracle_at_every_shape(libptap, port, golden_scene, shape):
+    """ptap_scene_build_grids against the oracle's restatement of Scene::addMeshesToGrid on non-cubic and thin grids."""
+    from pathtracerap_b200 import Scene
+    g = golden_scene
+    s = Scene.from_arrays(g["models"], g["meshes"], g["vertices"], g["triangles"])
+    s.build_grids(*shape)
+    a = s.arrays()
+    models, grids, voxels, refs = port.build_grids(g["models"], g["meshes"], g["vertices"], g["triangles"], shape)
+    assert a["grid_dim"] == shape
+    assert len(a["voxels"]) == len(grids) * int(np.prod(shape))
+    assert a["grids"].tobytes() == grids.tobytes()
+    assert a["voxels"].tobytes() == voxels.tobytes()
+    assert a["refs"].tobytes() == refs.tobytes()
+    assert np.array_equal(a["models"]["grid_index"], models["grid_index"])
+
+
+def _run_isolated(code, timeout=300):
+    """Runs `code` in a fresh interpreter at the repository root: a crash of the library is a failed test, not a dead pytest."""
+    return subprocess.run([sys.executable, "-c", textwrap.dedent(code)], cwd=ROOT, capture_output=True, text=True, timeout=timeout)
+
+
+# Two tiny triangles at opposite corners of their mesh's box: a handful of references at any grid size, so nothing but the dimension
+# checks stands between a grid whose cell count wraps and the cell loop.
+CORNERS_OBJ = "v 0 0 0\nv 0.01 0 0\nv 0 0.01 0\nv 0.1 0.1 0.1\nv 0.09 0.1 0.1\nv 0.1 0.09 0.1\nf 1 2 3\nf 4 5 6\n"
+# 2^21 and 2^22 per axis: each axis is within 2^27, and the product (2^63, 2^66) overflows a 64-bit product taken in one step
+WRAPPING_DIMS = [(2097152, 2097152, 2097152), (4194304, 4194304, 4194304)]
+
+
+@pytest.mark.parametrize("grid", ["[0, 25, 25]", "[-4, 25, 25]", "[4000, 4000, 4000]", "[1e10, 1, 1]"] + [str(list(d)) for d in WRAPPING_DIMS])
+def test_config_txt_bad_grid_is_a_parse_error(libptap, tmp_path, grid):
+    """GRID dimensions that are not positive, or whose product exceeds 2^27 cells (the limit of ptap_scene_build_grids, the product
+    included when it would overflow 64 bits), or that do not fit an int: PTAP_E_PARSE (-5) and "bad GRID"."""
+    (tmp_path / "corners.obj").write_text(CORNERS_OBJ)
+    cfg = tmp_path / "Config.txt"
+    cfg.write_text(f"MESH\ncorners\ncorners.obj\n\nGRID\n{grid}\n")
+    p = _run_isolated(f"""
+        import ctypes as C
+        from pathtracerap_b200 import _native as N
+        h = C.c_void_p()
+        print("rc", N.lib().ptap_scene_create_from_config({str(cfg)!r}.encode(), C.byref(h)), bool(h.value))
+    """)
+    assert p.returncode == 0, f"GRID {grid}: the process died ({p.returncode}): {p.stderr[-2000:]}"
+    assert "rc -5 False" in p.stdout and "bad GRID" in p.stderr, (p.stdout, p.stderr)
+
+
+@pytest.mark.parametrize("dims", WRAPPING_DIMS + [(1, 1, 1 << 27 | 1), (1 << 14, 1 << 14, 1)], ids=lambda d: "x".join(map(str, d)))
+def test_build_grids_refuses_dimensions_past_2p27_cells(libptap, tmp_path, dims):
+    """ptap_scene_build_grids with more than 2^27 cells - among them products that overflow 64 bits when taken in one step: PTAP_E_INVALID
+    and "bad grid dimensions", the scene's grids kept.  Run in a subprocess: a wrapped cell count would take the process down."""
+    (tmp_path / "corners.obj").write_text(CORNERS_OBJ)
+    p = _run_isolated(f"""
+        from pathtracerap_b200 import PtapError, Scene
+        s = Scene.empty()
+        s.add_model(s.add_obj({str(tmp_path / "corners.obj")!r}))
+        s.build_grids(3, 4, 5)
+        before = s.arrays()
+        try:
+            s.build_grids(*{dims!r})
+            print("accepted")
+        except PtapError as e:
+            print("refused:", e)
+        after = s.arrays()
+        print("kept", after["grid_dim"] == (3, 4, 5) and all(before[k].tobytes() == after[k].tobytes() for k in ("grids", "voxels", "refs")))
+    """)
+    assert p.returncode == 0, f"the process died ({p.returncode}): {p.stderr[-2000:]}"
+    assert "refused:" in p.stdout and "error -1" in p.stdout and "bad grid dimensions" in p.stdout and "kept True" in p.stdout, p.stdout
+
+
+def test_config_txt_non_cubic_grid(libptap, tmp_path):
+    from pathtracerap_b200 import Scene
+    (tmp_path / "one.obj").write_text("v 0 0 0\nv 1 0 0\nv 0 1 0\nv 1 1 0\nf 1 2 4 3\n")
+    cfg = tmp_path / "Config.txt"
+    cfg.write_text(CONFIG + "\nGRID\n[7, 40, 3]\n")
+    a = Scene(str(cfg)).arrays()
+    assert a["grid_dim"] == (7, 40, 3)
+    assert len(a["grids"]) == 3 and len(a["voxels"]) == 3 * 840
+
+
+def box_filling_mesh(s, copies):
+    """A mesh of `copies` coincident triangles whose bounding box is the mesh's: at 512^3 every one is listed in all 2^27 cells."""
+    from pathtracerap_b200 import VERTEX
+    v = np.zeros(3, VERTEX); v["position"] = [[0, 0, 0], [100, 100, 0], [0, 100, 100]]; v["normal"] = (0, 0, 1)
+    return s.add_mesh(v, np.tile(np.array([[0, 1, 2]], np.int32), (copies, 1)))
+
+
+@pytest.mark.parametrize("case", ["17_coincident", "17_meshes"])
+def test_host_grid_builder_refuses_32bit_overflow(libptap, case):
+    """17 * 2^27 references in one grid, or 17 grids of 2^27 cells: more than 2^31 - 1, which the voxels' and the reference list's int
+    positions cannot hold.  build_grids fails with a message that names the count, in well under a second (both counts are taken before
+    any per-cell work), and the scene keeps the grids it had."""
+    p = _run_isolated(f"""
+        import sys, time
+        sys.path.insert(0, "tests")
+        from pathtracerap_b200 import PtapError, Scene
+        from test_host import box_filling_mesh
+        s = Scene.empty()
+        if {case!r} == "17_coincident":
+            s.add_model(box_filling_mesh(s, 17))
+        else:
+            for _ in range(17):
+                s.add_model(box_filling_mesh(s, 1))
+        s.build_grids(3, 4, 5)
+        before = s.arrays()
+        t = time.time()
+        try:
+            s.build_grids(512, 512, 512)
+            print("accepted")
+        except PtapError as e:
+            print("refused in %.3f s:" % (time.time() - t), e)
+        after = s.arrays()
+        print("kept", after["grid_dim"] == (3, 4, 5) and all(before[k].tobytes() == after[k].tobytes() for k in ("models", "grids", "voxels", "refs")))
+    """, timeout=120)
+    assert p.returncode == 0, f"the process died ({p.returncode}): {p.stderr[-2000:]}"
+    out = p.stdout
+    assert "refused in" in out and "kept True" in out, out
+    assert float(out.split("refused in ")[1].split()[0]) < 1.0, out
+    want = str(17 * 2 ** 27) + (" references" if case == "17_coincident" else " cells")
+    assert want in out, out
+
+
 def test_compose_trs_matches_reference_matrices(libptap, golden_scene):
     """translate * rotate(Y) * scale and its glm::inverse, bit-equal to the matrices the reference's Scene.cpp computes."""
     from pathtracerap_b200 import Scene
